@@ -6,6 +6,7 @@ definition (SURVEY 8(d)); phase B runs on arg-min labels (the GCO stand-in of 8(
     python bench.py --gpus N --steps K --warmup W           # this repo, one process per GPU
     python bench.py --impl reference --steps K --warmup W   # the reference's CPU path
     python bench.py --workload cfg4_genome_50kb             # another BASELINE configuration
+    python bench.py --dump-outputs DIR                      # also write the last timed step's outputs as .npy
 
 A *step* is one pass of the hot path over every region (or row band) this rank holds: phase A1
 emission (+max|logp|), A2 integer unary + integer edge weights + per-node maxima, B fused
@@ -323,6 +324,13 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     launches = engine.launch_count() - launches0
     total_ms = t_start.elapsed_time(t_end)
+    # the last timed step's results, read before the untimed phase-timing steps below run the regions again
+    if world > 1 or single:
+        final = (stats_dev[0] if single else total_stats).cpu().numpy()
+    else:
+        final = sum(t_.cpu().numpy() for t_ in stats_dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, final, pieces, K, d)
     phase_ms = np.zeros(3)        # per step, summed over this rank's regions
     if single:
         for evs in all_evs:
@@ -363,10 +371,6 @@ def run_ours(args):
 
     # ---- correctness of what was timed: the posteriors of every node sum to one, so the first K
     # statistics (after the all-reduce) must add up to the number of nodes
-    if world > 1 or single:
-        final = (stats_dev[0] if single else total_stats).cpu().numpy()
-    else:
-        final = sum(t_.cpu().numpy() for t_ in stats_dev)
     post_sum = float(final[:K].sum())
     expect = nodes_total if world > 1 else float(n_rank)
     if not abs(post_sum - expect) <= 1e-6 * expect:
@@ -472,6 +476,50 @@ def run_ours(args):
     m.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+LOGPROB_SAMPLE_ROWS = 65536     # 15.7 MB of float64 at K=30
+
+
+def dump_outputs(out_dir, final, pieces, K, d):
+    """What the last timed step computed, as float64 .npy files for comparing two builds output for output
+    (the inputs are a pure function of SEED and the workload):
+
+    * stats_post, stats_obs, stats_obs_obsT, cost_sums: the statistics the step returns (summed over this
+      rank's regions and, for N>1, all-reduced) and its three cost sums;
+    * logprob_rows: the phase-A1 log-likelihood, a seeded sample of node rows of this rank's pieces
+      (logprob_index: piece, node);
+    * unary_i32_rows, w_i32, V_i32, dwf: what phase A2 hands to the graph cut -- the integer unary of the
+      same nodes, a seeded sample of the integer edge weights (w_index: piece, edge), the integer label
+      compatibility and the down-weight factor of each piece.  They are read back with phmrf_quantise,
+      which converts the log-likelihood the last step left on the device again; the conversion is exact
+      integer arithmetic on the same input, so these are the arrays the step computed."""
+    from phylo_hmrf_b200.engine import unpack_stats
+    os.makedirs(out_dir, exist_ok=True)
+    final = np.asarray(final, dtype=np.float64)
+    stats = unpack_stats(final, K, d)
+    arrays = {"stats_post": stats["post"], "stats_obs": stats["obs"], "stats_obs_obsT": stats["obs*obs.T"],
+              "cost_sums": final[-3:]}
+    rng = np.random.default_rng(SEED)
+    per_piece = max(1, LOGPROB_SAMPLE_ROWS // len(pieces))
+    out = {k: [] for k in ("logprob_rows", "logprob_index", "unary_i32_rows", "w_i32", "w_index", "V_i32", "dwf")}
+    for i, p in enumerate(pieces):
+        pick = np.sort(rng.choice(p.n, size=min(per_piece, p.n), replace=False))
+        lp = p.reg.logprob()
+        out["logprob_rows"].append(lp[pick])
+        out["logprob_index"].append(np.column_stack([np.full(len(pick), i), pick]))
+        del lp
+        q = p.reg.quantise(boundary_cap=0)
+        out["unary_i32_rows"].append(q["unary_i32"][pick])
+        edges = np.sort(rng.choice(p.E, size=min(per_piece, p.E), replace=False))
+        out["w_i32"].append(q["w_i32"][edges])
+        out["w_index"].append(np.column_stack([np.full(len(edges), i), edges]))
+        out["V_i32"].append(q["V_i32"][None])
+        out["dwf"].append([q["dwf"]])
+        del q
+    arrays.update({k: np.concatenate(v) for k, v in out.items()})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def run_e2e(args, torch, dist, ph, m, pieces, d, K, world, stats_len):
@@ -722,7 +770,11 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--e2e-trace", action="store_true", help="per-call wall times of the end-to-end passes on stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

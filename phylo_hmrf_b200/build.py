@@ -4,11 +4,8 @@
 
 * ``lib/libphmrf.so``      hand-written CUDA kernels + the C ABI of include/phmrf.h
 * ``lib/libphmrf_probe.so``  pipe probes for the roofline denominators (bench/tools only; include/phmrf_probe.h)
-* ``lib/libphmrf_gco.so``  thin C wrapper (csrc/gco_wrap.cpp, include/phmrf_gco.h) around the
-  GCO v3.0 graph-cut library.  GCO is third-party code that the reference vendors under
-  ``gco_source/``; it is compiled from where it lies (``$PHMRF_GCO_SRC``, default
-  ``/root/reference/gco_source``) and never copied into this repository.  When the source
-  tree is absent (e.g. on the GPU box) a previously built ``.so`` is used as is.
+* ``lib/libphmrf_gco.so``  host graph cut (csrc/gco.cpp, include/phmrf_gco.h): GCO v3.0's
+  alpha-beta swap and alpha-expansion on a general graph
 """
 from __future__ import annotations
 
@@ -24,8 +21,6 @@ LIB = os.path.join(PKG, "lib")
 OBJ = os.path.join(PKG, "build")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 CU_SOURCES = ["api.cu", "kernels_a.cu", "kernels_b.cu", "kernels_b3.cu", "kernels_b3_d58.cu", "kernels_b3_d9c.cu", "kernels_grid.cu", "kernels_prep.cu"]
-GCO_SRC = os.environ.get("PHMRF_GCO_SRC", "/root/reference/gco_source")
-GCO_FILES = ["GCoptimization.cpp", "LinkedBlockList.cpp"]
 
 
 def _nvcc() -> str:
@@ -94,15 +89,11 @@ def build_probe(force=False):
 def build_gco(force=False):
     os.makedirs(LIB, exist_ok=True)
     out = os.path.join(LIB, "libphmrf_gco.so")
-    wrap = os.path.join(CSRC, "gco_wrap.cpp")
-    gco = [os.path.join(GCO_SRC, f) for f in GCO_FILES]
-    if not all(os.path.exists(f) for f in gco):
-        if os.path.exists(out):
-            return out  # GPU box: prebuilt library travels with the snapshot
-        raise RuntimeError("GCO v3.0 sources not found under %s (set PHMRF_GCO_SRC)" % GCO_SRC)
-    if not force and not _newer(out, [wrap] + gco):
+    src = os.path.join(CSRC, "gco.cpp")
+    hdr = os.path.join(PKG, "..", "include", "phmrf_gco.h")
+    if not force and not _newer(out, [src, hdr]):
         return out
-    _run(["g++", "-O2", "-w", "-fPIC", "-shared", "-std=gnu++17", "-I", GCO_SRC, "-o", out, wrap] + gco)
+    _run(["g++", "-O2", "-Wall", "-fPIC", "-shared", "-std=gnu++17", "-o", out, src])
     return out
 
 

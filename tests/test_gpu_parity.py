@@ -125,7 +125,7 @@ def test_dropin_class_matches_reference_queue_tuple(ph, golden):
         assert model._predict_posteriors(X, len_vec, r, q) is True
         rid, stats, labels, c_pair, c_pn, c_un, c_tot = q.items[-1]
         assert rid == r
-        # label identity: oracle integer arrays -> same vendored GCO -> same labels
+        # label identity: oracle integer arrays -> same graph cut -> same labels
         lp_ref = golden[p + "logprob"]
         u_ref, w_ref, V_ref, _ = orc.pygco_quantise(-lp_ref, golden[p + "ref_edge_w"], golden["ref_V"])
         qd = model.last_quantise

@@ -90,32 +90,3 @@ def test_quantiles_match_the_reference(tmp_path):
     dirs = write_loader_inputs(str(tmp_path), G)
     q = loader.quantile_contact_vec(["3"], int(G["resolution"]), str(tmp_path / "chrom.sizes"), dirs, SPECIES)
     np.testing.assert_array_equal(q, G["quantiles"])
-
-
-def test_alignment_on_the_reference_example_data():
-    """Where the reference tree is present (build container): its own multi_contact_matrix3A, executed
-    through ref_loader on the shipped chr22 files of three species, against loader.multi_contact_matrix3A."""
-    import math
-    import pandas as pd
-    import ref_loader
-    root = os.path.join(ref_loader.REF, "example_input")
-    dirs = [os.path.join(root, "test_data", d) for d in ("hic_gorGor4", "hic_panTro5", "hic_panPan2")]
-    if not ref_loader.available() or not all(os.path.exists(os.path.join(d, "chr22.50K.txt")) for d in dirs):
-        pytest.skip("reference example data not present")
-    from phylo_hmrf_b200 import loader
-    patches = [("math.ceil(chrom_size/resolution)", "math.ceil(chrom_size//resolution)"),
-               ("x1, x2 = x1/resolution, x2/resolution", "x1, x2 = x1//resolution, x2//resolution"),
-               ("np.asarray(data2[2])", "np.array(data2[2])")]
-    util = ref_loader.load_utility(["mapping_Idx", "output_multi_contactMtx", "multi_contact_matrix3A"], patches)
-    util.update({"pd": pd, "math": math, "os": os})
-    species = ["gorGor4", "panTro5", "panPan2"]
-    sizes = os.path.join(root, "hg38.chrom.sizes")
-    ref = util["multi_contact_matrix3A"]("22", 50000, sizes, dirs, species, "", 0)
-    got = loader.multi_contact_matrix3A("22", 50000, sizes, dirs, species, "", 0)
-    assert list(got) == list(ref) and len(got) == len(ref) > 100000
-    for c in list(ref):
-        np.testing.assert_array_equal(np.asarray(got[c]), np.asarray(ref[c]))
-    q_ref_fn = ref_loader.load_utility(["multi_contact_matrix3A_single", "quantile_contact"], patches)
-    q_ref_fn.update({"pd": pd, "math": math, "os": os})
-    np.testing.assert_array_equal(loader.quantile_contact("22", 50000, sizes, dirs, species),
-                                  q_ref_fn["quantile_contact"]("22", 50000, sizes, dirs, species))

@@ -177,6 +177,25 @@ int phmrf_estep_stats_async(phmrf_region *r, int estimate_type);
 /* Number of kernel launches this library has enqueued so far (bench "gpu_launches"). */
 int64_t phmrf_launch_count(void);
 
+/* ------------------------------------------------------------------ graph cut ----------- */
+
+/* The alpha-beta swap of csrc/gco.cpp (phmrf_gco_cut_general_graph with algorithm PHMRF_GCO_SWAP) on the
+ * device, host arrays in, with the same meaning.  Same labels and energies as the host cut: every move takes
+ * the smallest sink side of all minimum cuts, which depends on the energy alone.  Sites are indexed with 64
+ * bits (no n_sites*n_labels < 2^31 limit).  Errors where the host returns one (a term above
+ * GCO_MAX_ENERGYTERM in an executed move, a bad init label, edges not 0 <= id1 < id2 < n_sites);
+ * PHMRF_E_UNSUPPORTED for a negative edge weight or V[a][b] + V[b][a] < V[a][a] + V[b][b] (non-submodular
+ * moves, which only the host cut runs). */
+int phmrf_graph_cut_swap(int device, int64_t n_sites, int32_t n_labels, const int32_t *unary, const int64_t *edge_ids,
+                         const int32_t *edge_w, int64_t n_edges, const int32_t *smooth, const int32_t *init_labels,
+                         int32_t n_iter, int32_t *labels_out, long long *energy_out, long long *energy_before_out);
+/* The same on a whole region's own integer arrays from the last phmrf_quantise (unary, edge weights and V_i32):
+ * nothing crosses PCIe but the init labels (NULL: all 0) and, if labels_out != NULL, the result.  The labels
+ * stay resident for phmrf_estep_stats.  A band (n_own != n_window) is PHMRF_E_INVALID.  The region's cut scratch
+ * is allocated at its first call and counted in phmrf_region_device_bytes. */
+int phmrf_region_graph_cut(phmrf_region *r, const int32_t *init_labels, int32_t n_iter, int32_t *labels_out,
+                           long long *energy_out, long long *energy_before_out);
+
 /* ------------------------------------------------------------------ next row (f-1) ---- */
 
 /* utility.py:1871-1973 (edge_weightlist_grid3_undirected_unsym, kind=1: diagonal region of

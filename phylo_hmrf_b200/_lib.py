@@ -73,7 +73,12 @@ SIGNATURES = {
     "phmrf_region_own_offset": (C.c_int64, [_vp]),
     "phmrf_region_edges": (C.c_int, [_vp, _c_int64_p, _c_double_p]),
     "phmrf_region_set_edge_weights": (C.c_int, [_vp, _c_double_p, C.c_int64]),
-    "phmrf_grid_edge_count": (C.c_int64, [C.c_int, C.c_int64, C.c_int64, C.c_int]),
+    "phmrf_graph_cut_swap": (C.c_int, [C.c_int, C.c_int64, C.c_int32, _c_int32_p, _c_int64_p, _c_int32_p, C.c_int64,
+                                       _c_int32_p, _c_int32_p, C.c_int32, _c_int32_p, C.POINTER(C.c_longlong),
+                                       C.POINTER(C.c_longlong)]),
+    "phmrf_region_graph_cut": (C.c_int, [_vp, _c_int32_p, C.c_int32, _c_int32_p, C.POINTER(C.c_longlong),
+                                         C.POINTER(C.c_longlong)]),
+    "phmrf_grid_edge_count":(C.c_int64, [C.c_int, C.c_int64, C.c_int64, C.c_int]),
     "phmrf_grid_edges": (C.c_int, [C.c_int, _c_double_p, C.c_int, C.c_int, C.c_int64, C.c_int64, C.c_int, _c_double_p,
                                    C.c_int64]),
     "phmrf_prep_normalise": (C.c_int, [C.c_int, _c_double_p, C.c_int64, C.c_int, _c_double_p, _c_double_p, _c_double_p,

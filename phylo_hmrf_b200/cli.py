@@ -86,6 +86,11 @@ def run(opts, device=0):
     """phylo_hmrf.py:1570-1749.  Returns the dict written to the `.mat` file."""
     import scipy.io
     from .hmrf import phyloHMRF
+    # the graph cut of every EM iteration: 'host' (csrc/gco.cpp, default) or 'device' (the same swap on the GPU);
+    # an environment variable, so that the option list stays the reference's
+    graph_cut = os.environ.get("PHMRF_GRAPH_CUT", "host")
+    if graph_cut not in ("host", "device"):
+        raise SystemExit("PHMRF_GRAPH_CUT must be 'host' or 'device', not %r" % graph_cut)
     device, rank, world, td = _launch_context(device)
     run_id, K = int(opts.run_id), int(opts.num_states)
     cons_param = float(opts.cons_param)
@@ -125,7 +130,8 @@ def run(opts, device=0):
                       beta1=float(opts.beta1), initial_mode=int(opts.initial_mode),
                       initial_weight=float(opts.initial_weight), initial_weight1=float(opts.initial_weight1),
                       initial_magnitude=float(opts.initial_magnitude), learning_rate=0.001,
-                      estimate_type=int(opts.estimate_type), max_iter=100, n_iter=5000, tol=1e-7, device=device)
+                      estimate_type=int(opts.estimate_type), max_iter=100, n_iter=5000, tol=1e-7, device=device,
+                      graph_cut=graph_cut)
     filename = "%s/estimate_ou_%d_%.2f_%d_%s" % (output_path, run_id, cons_param, K, str(opts.annotation))
     res = model.fit_accumulate_test(samples, len_vec, float(opts.threshold), filename, int(opts.miter))
     params_vec1, params_vec2, params_vecList, iter_id1, iter_id2, cost_vec, state_vec = res

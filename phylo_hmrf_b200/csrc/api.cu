@@ -86,6 +86,8 @@ struct phmrf_region {
     double *d_scratch = nullptr;  // [K][ld] posteriors / AoS staging, allocated on demand
     int64_t scratch_elems = 0;
     bool have_logp = false, have_unary = false, have_labels = false, have_rowmax = false;
+    bool edges_sorted = true;   // edge list sorted by (id1, id2): the device cut numbers the edges from the slots
+    SwapScratch *cut = nullptr; // device graph cut, allocated at the first phmrf_region_graph_cut
     int64_t bytes = 0;
     // small results (statistics, flags, dwf, counters) come back through a host-mapped buffer that a
     // kernel writes (launch_publish), not through the copy engines
@@ -332,12 +334,15 @@ int phmrf_region_create(phmrf_ctx *ctx, const double *X, int64_t n_own, int64_t 
     // ---- graph layout on the host: per owned node, its neighbours in ascending edge order
     std::vector<int> deg((size_t)n_own, 0);
     double wmax = 0.0;
+    bool sorted = true;
     for (int64_t e = 0; e < n_edges; ++e) {
         const int64_t a = edge_ids[2 * e], b = edge_ids[2 * e + 1];
         if (a < 0 || b < 0 || a >= n_window || b >= n_window || a == b) {
             set_error("phmrf_region_create: edge id out of range (or self loop) at edge " + std::to_string(e));
             return PHMRF_E_INVALID;
         }
+        if (a > b || (e > 0 && (edge_ids[2 * e - 2] > a || (edge_ids[2 * e - 2] == a && edge_ids[2 * e - 1] > b))))
+            sorted = false;
         if (a >= own_offset && a < own_offset + n_own) deg[a - own_offset]++;
         if (b >= own_offset && b < own_offset + n_own) deg[b - own_offset]++;
         const double aw = std::fabs(edge_w[e]);
@@ -354,6 +359,7 @@ int phmrf_region_create(phmrf_ctx *ctx, const double *X, int64_t n_own, int64_t 
     r->E = n_edges;
     r->W = W;
     r->wmax = wmax;
+    r->edges_sorted = sorted;
     r->ld = round_up(n_own > 0 ? n_own : 1, 64);
     if (stream) {
         r->stream = (cudaStream_t)stream;
@@ -651,6 +657,10 @@ int phmrf_region_destroy(phmrf_region *r) {
     cudaFree(r->d_flags);
     cudaFree(r->d_badlabel);
     cudaFree(r->d_scratch);
+    if (r->cut) {
+        swap_scratch_free(*r->cut);
+        delete r->cut;
+    }
     if (r->h_small) cudaFreeHost(r->h_small);
     if (r->own_stream) cudaStreamDestroy(r->stream);
     cudaGetLastError();
@@ -970,6 +980,130 @@ int phmrf_set_logprob(phmrf_region *r, const double *logprob) {
     r->have_logp = true;
     r->have_unary = false;
     r->have_rowmax = true;
+    return PHMRF_OK;
+}
+
+// ---------------------------------------------------------------- graph cut on the device
+int phmrf_graph_cut_swap(int device, int64_t n_sites, int32_t n_labels, const int32_t *unary, const int64_t *edge_ids,
+                         const int32_t *edge_w, int64_t n_edges, const int32_t *smooth, const int32_t *init_labels,
+                         int32_t n_iter, int32_t *labels_out, long long *energy_out, long long *energy_before_out) {
+    if (n_sites <= 0 || n_labels <= 0 || !unary || !smooth || !labels_out || n_edges < 0 ||
+        (n_edges > 0 && (!edge_ids || !edge_w))) {
+        set_error("GCO (device swap) phmrf_graph_cut_swap: invalid arguments");
+        return PHMRF_E_INVALID;
+    }
+    for (int64_t e = 0; e < n_edges; ++e) {
+        const int64_t a = edge_ids[2 * e], b = edge_ids[2 * e + 1];
+        if (a < 0 || b < 0 || a >= n_sites || b >= n_sites || a >= b) {
+            set_error("GCO (device swap) phmrf_graph_cut_swap: edges must satisfy 0 <= id1 < id2 < n_sites");
+            return PHMRF_E_INVALID;
+        }
+    }
+    if (init_labels)
+        for (int64_t i = 0; i < n_sites; ++i)
+            if (init_labels[i] < 0 || init_labels[i] >= n_labels) {
+                set_error("GCO (device swap) phmrf_graph_cut_swap: init label out of range");
+                return PHMRF_E_INVALID;
+            }
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || device < 0 || device >= count) {
+        cudaGetLastError();
+        set_error("GCO (device swap) phmrf_graph_cut_swap: no such CUDA device (this library has no CPU fallback)");
+        return PHMRF_E_CUDA;
+    }
+    PHMRF_CUDA(cudaSetDevice(device));
+    cudaStream_t st = nullptr;
+    PHMRF_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+    SwapScratch s;
+    int32_t *d_unary = nullptr, *d_w = nullptr, *d_labels = nullptr;
+    long long *d_ids = nullptr;
+    int rc = swap_scratch_alloc(s, n_sites, n_edges, n_labels);
+    const size_t nu = sizeof(int32_t) * (size_t)n_sites * n_labels;
+    if (rc == PHMRF_OK &&
+        (cudaMalloc((void **)&d_unary, nu) != cudaSuccess ||
+         cudaMalloc((void **)&d_labels, sizeof(int32_t) * n_sites) != cudaSuccess ||
+         cudaMalloc((void **)&d_w, sizeof(int32_t) * (n_edges > 0 ? n_edges : 1)) != cudaSuccess ||
+         cudaMalloc((void **)&d_ids, sizeof(long long) * 2 * (n_edges > 0 ? n_edges : 1)) != cudaSuccess ||
+         cudaMemcpyAsync(d_unary, unary, nu, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+         (n_edges > 0 &&
+          (cudaMemcpyAsync(d_w, edge_w, sizeof(int32_t) * n_edges, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+           cudaMemcpyAsync(d_ids, edge_ids, sizeof(long long) * 2 * n_edges, cudaMemcpyHostToDevice, st) !=
+               cudaSuccess)) ||
+         (init_labels ? cudaMemcpyAsync(d_labels, init_labels, sizeof(int32_t) * n_sites, cudaMemcpyHostToDevice, st)
+                      : cudaMemsetAsync(d_labels, 0, sizeof(int32_t) * n_sites, st)) != cudaSuccess))
+        rc = cuda_fail(cudaGetLastError(), "graph cut upload", __FILE__, __LINE__);
+    if (rc == PHMRF_OK) rc = swap_graph_from_edges(s, d_ids, st);
+    if (rc == PHMRF_OK) rc = swap_run(s, d_unary, d_w, smooth, d_labels, n_iter, energy_out, energy_before_out, st);
+    if (rc == PHMRF_OK &&
+        (cudaMemcpyAsync(labels_out, d_labels, sizeof(int32_t) * n_sites, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+         cudaStreamSynchronize(st) != cudaSuccess))
+        rc = cuda_fail(cudaGetLastError(), "graph cut download", __FILE__, __LINE__);
+    cudaStreamSynchronize(st);
+    cudaFree(d_unary);
+    cudaFree(d_labels);
+    cudaFree(d_w);
+    cudaFree(d_ids);
+    swap_scratch_free(s);
+    cudaStreamDestroy(st);
+    return rc;
+}
+
+int phmrf_region_graph_cut(phmrf_region *r, const int32_t *init_labels, int32_t n_iter, int32_t *labels_out,
+                           long long *energy_out, long long *energy_before_out) {
+    if (!r) return PHMRF_E_INVALID;
+    if (r->n != r->n_window || r->n == 0) {
+        set_error("GCO (device swap) phmrf_region_graph_cut: needs a whole, non-empty region (a band's cut needs the other bands' unary)");
+        return PHMRF_E_INVALID;
+    }
+    if (!r->edges_sorted) {
+        set_error("GCO (device swap) phmrf_region_graph_cut: the region's edge list is not sorted by (id1, id2)");
+        return PHMRF_E_INVALID;
+    }
+    if (!r->have_unary) {
+        set_error("GCO (device swap) phmrf_region_graph_cut: call phmrf_quantise first");
+        return PHMRF_E_STATE;
+    }
+    phmrf_ctx *ctx = r->ctx;
+    int rc = set_device(ctx);
+    if (rc) return rc;
+    const int K = ctx->K;
+    if (!r->cut) {
+        r->cut = new SwapScratch();
+        rc = swap_scratch_alloc(*r->cut, r->n, r->E, K);
+        if (rc == PHMRF_OK) rc = swap_graph_from_ell(*r->cut, r->d_nbr_id, r->W, r->ld, r->stream);
+        if (rc == PHMRF_OK) PHMRF_CUDA(cudaStreamSynchronize(r->stream));
+        if (rc != PHMRF_OK) {
+            swap_scratch_free(*r->cut);
+            delete r->cut;
+            r->cut = nullptr;
+            return rc;
+        }
+        r->bytes += r->cut->bytes;
+    }
+    r->have_labels = false;
+    if (init_labels) {
+        PHMRF_CUDA(cudaMemcpyAsync(r->d_labels, init_labels, sizeof(int32_t) * r->n, cudaMemcpyHostToDevice, r->stream));
+        if ((rc = launch_check_labels(r->d_labels, r->n, K, r->d_badlabel, r->stream)) != PHMRF_OK) return rc;
+        if ((rc = launch_publish(r->d_small + kSmBadLabel, r->d_badlabel, 1, false, r->stream)) != PHMRF_OK) return rc;
+        PHMRF_CUDA(cudaStreamSynchronize(r->stream));
+        const long long first_bad = (long long)r->h_small[kSmBadLabel];
+        if (first_bad >= 0) {
+            set_error("GCO (device swap) phmrf_region_graph_cut: init label out of range at node " + std::to_string(first_bad));
+            return PHMRF_E_INVALID;
+        }
+    } else {
+        PHMRF_CUDA(cudaMemsetAsync(r->d_labels, 0, sizeof(int32_t) * r->n, r->stream));
+    }
+    std::vector<int32_t> V((size_t)K * K);  // as phmrf_quantise hands V_i32 to the host cut
+    for (int i = 0; i < K * K; ++i) V[i] = (int32_t)(ctx->V[i] * ctx->sprec);
+    if ((rc = swap_run(*r->cut, r->d_unary, r->d_edge_wi, V.data(), r->d_labels, n_iter, energy_out, energy_before_out,
+                       r->stream)) != PHMRF_OK)
+        return rc;
+    if (labels_out) {
+        PHMRF_CUDA(cudaMemcpyAsync(labels_out, r->d_labels, sizeof(int32_t) * r->n, cudaMemcpyDeviceToHost, r->stream));
+        PHMRF_CUDA(cudaStreamSynchronize(r->stream));
+    }
+    r->have_labels = true;
     return PHMRF_OK;
 }
 

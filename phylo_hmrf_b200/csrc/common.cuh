@@ -141,4 +141,32 @@ int launch_band_fwd(const double *Xw_dev, int kind, long long n1, long long n2, 
                     long long n_fw, double beta1, long long ldw, double2 *fwd, cudaStream_t s);
 int launch_fwd_factor(double2 *fwd, long long count, double beta, int weighted, cudaStream_t s);
 
+// ---- alpha-beta swap on the device (kernels_cut.cu) ---------------------------------------
+// The graph in CSR form (both directions of every edge; per slot its edge number and the slot of the
+// reverse arc) and the max-flow arrays of one move, for n sites, E edges and K labels.  About
+// 52 bytes per site and 36 per slot (2E slots).
+struct SwapScratch {
+    int64_t n = 0, E = 0, bytes = 0;
+    int K = 0;
+    long long *start = nullptr;                                       // [n+1]
+    long long *nbr = nullptr, *eid = nullptr, *rev = nullptr, *rcap = nullptr;  // [2E]
+    int32_t *wslot = nullptr;                                         // [2E] integer edge weight per slot
+    long long *act = nullptr, *var = nullptr;                         // active sites; site -> compact index or -1
+    long long *excess = nullptr, *inflow = nullptr, *tcap = nullptr;  // per compact index
+    int *h = nullptr;                                                 // heights
+    int32_t *V = nullptr;                                             // [K*K]
+    long long *ctl = nullptr;                                         // control words
+    unsigned long long *h_map = nullptr, *d_map = nullptr;            // their host-mapped copy
+};
+int swap_scratch_alloc(SwapScratch &s, int64_t n, int64_t E, int K);
+void swap_scratch_free(SwapScratch &s);
+// the graph from a device edge list [E,2] (0 <= id1 < id2 < n)
+int swap_graph_from_edges(SwapScratch &s, const long long *edge_ids, cudaStream_t st);
+// the graph from a region's neighbour slots [W][ld] (-1 = empty), filled from an edge list sorted by (id1, id2)
+int swap_graph_from_ell(SwapScratch &s, const int32_t *nbr_id, int W, int64_t ld, cudaStream_t st);
+// GeneralGraphCut::swap(n_iter) of csrc/gco.cpp on device arrays: unary [n][K], w_edge [E], labels [n] (in: the
+// start, out: the result); V_host [K*K].  PHMRF_E_UNSUPPORTED for negative weights or a non-submodular V.
+int swap_run(SwapScratch &s, const int32_t *unary, const int32_t *w_edge, const int32_t *V_host, int32_t *labels,
+             int n_iter, long long *energy_out, long long *energy_before_out, cudaStream_t st);
+
 }  // namespace phmrf

@@ -185,6 +185,22 @@ class Region:
         check(_lib.lib().phmrf_labels_argmin_unary(self._h, i32ptr(out)))
         return out
 
+    def graph_cut(self, init_labels=None, n_iter=5000, return_energy=False):
+        """Alpha-beta swap on the region's own integer arrays from the last quantise() (phmrf_region_graph_cut):
+        the labels of gco_cut_int(..., algorithm='swap') on those arrays, without downloading them.  The labels
+        stay on the device for estep_stats(); they are also returned (with the energy after and before the cut
+        when return_energy).  Whole regions only."""
+        init = None
+        if init_labels is not None:
+            init = np.ascontiguousarray(init_labels, dtype=np.int32)
+            if init.shape != (self.n,):
+                raise ValueError("init_labels must hold %d labels" % self.n)
+        out = np.empty(self.n, dtype=np.int32)
+        en, en0 = C.c_longlong(), C.c_longlong()
+        check(_lib.lib().phmrf_region_graph_cut(self._h, i32ptr(init), int(n_iter), i32ptr(out), C.byref(en),
+                                                C.byref(en0)))
+        return (out, en.value, en0.value) if return_energy else out
+
     def estep_stats(self, estimate_type, want_post=False):
         """-> (stats dict like phylo_hmrf.py:311-314, cost_sums[3], posteriors or None)"""
         K, d = self.model.K, self.model.d
@@ -338,6 +354,35 @@ def gco_cut_int(unary_i32, edge_ids, w_i32, V_i32, n_iter=-1, algorithm='expansi
                                        int(n_iter), alg, i32ptr(out), C.byref(en), C.byref(en0))
     if rc != 0:
         raise RuntimeError(g.phmrf_gco_last_error().decode("utf-8", "replace"))
+    return (out, en.value, en0.value) if return_energy else out
+
+
+def swap_supported(V_i32, w_min):
+    """True when the device swap runs these costs: no negative edge weight and V[a][b] + V[b][a] >=
+    V[a][a] + V[b][b] for every pair of labels, so that every swap move is submodular.  The host cut also runs
+    the other cases (with negative capacities)."""
+    V = np.asarray(V_i32, dtype=np.int64)
+    d = np.diag(V)
+    return bool(w_min >= 0 and np.all(V + V.T >= d[:, None] + d[None, :]))
+
+
+def gco_swap_device(unary_i32, edge_ids, w_i32, V_i32, n_iter=-1, init_labels=None, return_energy=False, device=0):
+    """gco_cut_int(..., algorithm='swap') on the GPU (phmrf_graph_cut_swap): the same labels and energies.
+    Costs swap_supported() refuses raise PhmrfError with code PHMRF_E_UNSUPPORTED."""
+    u = np.ascontiguousarray(unary_i32, dtype=np.int32)
+    n, K = u.shape
+    e = np.ascontiguousarray(edge_ids, dtype=np.int64).reshape(-1, 2)
+    w = np.ascontiguousarray(w_i32, dtype=np.int32)
+    V = np.ascontiguousarray(V_i32, dtype=np.int32)
+    if len(w) != len(e) or V.shape != (K, K):
+        raise ValueError("need w_i32 [%d] and V_i32 [%d, %d]" % (len(e), K, K))
+    init = None if init_labels is None else np.ascontiguousarray(init_labels, dtype=np.int32)
+    if init is not None and init.shape != (n,):
+        raise ValueError("init_labels must hold %d labels" % n)
+    out = np.empty(n, dtype=np.int32)
+    en, en0 = C.c_longlong(), C.c_longlong()
+    check(_lib.lib().phmrf_graph_cut_swap(int(device), n, K, i32ptr(u), i64ptr(e), i32ptr(w), len(e), i32ptr(V),
+                                          i32ptr(init), int(n_iter), i32ptr(out), C.byref(en), C.byref(en0)))
     return (out, en.value, en0.value) if return_energy else out
 
 

@@ -49,6 +49,7 @@ class _IncidentEdges:
 
 class phyloHMRF(object):
     """Hot-path subset of the reference's ``phyloHMRF(_BaseGraph)`` (phylo_hmrf.py:51-150)."""
+    graph_cut = 'host'     # see __init__
 
     def __init__(self, n_samples, n_features, edge_list=None, branch_list=None, cons_param=1, beta=1.0, beta1=0.5,
                  initial_mode=0, initial_weight=0.3, initial_weight1=0.1, initial_magnitude=1, observation=None,
@@ -56,9 +57,16 @@ class phyloHMRF(object):
                  covariance_type='full', min_covar=1e-3, startprob_prior=1.0, transmat_prior=1.0, means_prior=0,
                  means_weight=0, covars_prior=1e-2, covars_weight=1, algorithm="viterbi", random_state=None,
                  n_iter=10, tol=1e-2, verbose=False, params="stmc", init_params="stmc", learning_rate=0.001,
-                 device=0, implicit_grid=True):
+                 device=0, implicit_grid=True, graph_cut='host'):
         if covariance_type != 'full':
             raise ValueError("the device path implements covariance_type='full' (phylo_hmrf.py:57)")
+        if graph_cut not in ('host', 'device'):
+            raise ValueError("graph_cut must be 'host' or 'device'")
+        # 'host': the integer costs are downloaded and cut by csrc/gco.cpp, and last_quantise holds every integer
+        # array.  'device': the same swap runs on the GPU on the region's own arrays (same labels), nothing but the
+        # labels crosses PCIe, and last_quantise holds dwf and V_i32 only.  Costs the device cut does not run
+        # (negative edge weights, non-submodular V) still go to the host.
+        self.graph_cut = graph_cut
         self.n_components = int(n_components)
         self.n_features = int(n_features)
         self.n_samples = int(n_samples)
@@ -213,27 +221,49 @@ class phyloHMRF(object):
         finally:
             reg.close()
 
+    def _device_cut(self, edge_w):
+        """Whether graph_cut='device' applies to these costs (engine.swap_supported on the V_i32 the quantiser
+        makes and the sign of the edge weights, both known on the host)."""
+        if self.graph_cut != 'device':
+            return False
+        V_i32 = (np.asarray(self.edge_potential, dtype=np.float64) * self._model.quantiser()[2]).astype(np.int32)
+        w = np.asarray(edge_w)
+        return engine.swap_supported(V_i32, float(w.min()) if len(w) else 0.0)
+
     def _estimate_state_graphcuts_gco(self, X, init_labels1, edge_idList_undirected, edge_weightList_undirected,
                                       want_logprob=True, staged_labels=False):
         """phylo_hmrf.py:486-507: emission, integer cost arrays (GPU), alpha-beta swap with
-        5000 cycles from ``init_labels1`` (host GCO).  Returns (labels, logprob)."""
+        5000 cycles from ``init_labels1`` (host GCO, or the GPU with graph_cut='device').  Returns (labels, logprob)."""
+        return self._graph_cut(X, init_labels1, edge_idList_undirected, edge_weightList_undirected, want_logprob,
+                               staged_labels)[:2]
+
+    def _graph_cut(self, X, init_labels1, edge_idList_undirected, edge_weightList_undirected, want_logprob=True,
+                   staged_labels=False):
+        """_estimate_state_graphcuts_gco -> (labels, logprob, the resident region that holds the labels on the
+        device, or None)."""
         self._sync_model()
         reg, temp = self._region_for(X, edge_idList_undirected, edge_weightList_undirected)
         try:
             reg.emit_loglik()
-            # resident regions keep page-locked staging buffers: the integer arrays go straight from the
-            # device into the graph cut, and its labels straight back (no pageable copies in between)
-            q = reg.quantise(staged=not temp)
             max_cycles1 = 5000
-            labels = engine.gco_cut_int(q["unary_i32"], edge_idList_undirected, q["w_i32"], q["V_i32"],
-                                        n_iter=max_cycles1, algorithm='swap', init_labels=init_labels1,
-                                        out=None if temp else reg.label_staging())
-            self.last_quantise = q
+            on_device = self._device_cut(edge_weightList_undirected)
+            if on_device:
+                q = reg.quantise(want_unary=False, want_edges=False)
+                labels = reg.graph_cut(init_labels1, n_iter=max_cycles1)
+                self.last_quantise = dict(dwf=q["dwf"], V_i32=q["V_i32"])
+            else:
+                # resident regions keep page-locked staging buffers: the integer arrays go straight from the
+                # device into the graph cut, and its labels straight back (no pageable copies in between)
+                q = reg.quantise(staged=not temp)
+                labels = engine.gco_cut_int(q["unary_i32"], edge_idList_undirected, q["w_i32"], q["V_i32"],
+                                            n_iter=max_cycles1, algorithm='swap', init_labels=init_labels1,
+                                            out=None if temp else reg.label_staging())
+                self.last_quantise = q
+                if not temp and not staged_labels:
+                    labels = labels.copy()     # the staging buffer is overwritten by the region's next graph cut
             logprob = reg.logprob() if want_logprob else None
             reg._host_logprob = logprob
-            if not temp and not staged_labels:
-                labels = labels.copy()     # the staging buffer is overwritten by the region's next graph cut
-            return labels, logprob
+            return labels, logprob, reg if on_device and not temp else None
         finally:
             if temp:
                 reg.close()
@@ -312,10 +342,11 @@ class phyloHMRF(object):
         s1, s2 = int(lv[1]), int(lv[2])
         reg = self._regions[region_id]
         init_labels = self.labels_local[s1:s2].copy()
-        labels, _ = self._estimate_state_graphcuts_gco(
+        labels, _, resident = self._graph_cut(
             X[s1:s2], init_labels, self.edge_idList_undirected_vec[region_id],
             self.edge_weightList_undirected_vec[region_id], want_logprob=False, staged_labels=True)
-        reg.set_labels(labels)
+        if resident is not reg:      # the device cut left its labels on the region already
+            reg.set_labels(labels)
         stats, sums, _ = reg.estep_stats(self.estimate_type)
         c = engine.costs_from_sums(sums, reg.n)
         m_queue.put((region_id, stats, labels, c[0], c[1], c[2], c[3]))
@@ -467,8 +498,12 @@ class phyloHMRF(object):
         labels = None
         if comm.rank == owner:
             w_i32, V_i32 = self._region_edge_costs(rid, dwf)
-            labels = engine.gco_cut_int(unary, self.edge_idList_undirected_vec[rid], w_i32, V_i32, n_iter=5000,
-                                        algorithm='swap', init_labels=self.labels_local[s1:s2].copy())
+            if self._device_cut(w):
+                labels = engine.gco_swap_device(unary, self.edge_idList_undirected_vec[rid], w_i32, V_i32, n_iter=5000,
+                                                init_labels=self.labels_local[s1:s2].copy(), device=self.device)
+            else:
+                labels = engine.gco_cut_int(unary, self.edge_idList_undirected_vec[rid], w_i32, V_i32, n_iter=5000,
+                                            algorithm='swap', init_labels=self.labels_local[s1:s2].copy())
         # label windows back to the bands, E-step per band
         n_stat = K * (1 + self.n_features + self.n_features * self.n_features)
         part = np.zeros(n_stat + 3)

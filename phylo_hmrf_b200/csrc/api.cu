@@ -834,8 +834,9 @@ int phmrf_labels_argmin_unary(phmrf_region *r, int32_t *labels_out) {
     return PHMRF_OK;
 }
 
+// overflow_redo: the redo after the pipeline kernel flagged a soft-max overflow, always on the general kernel
 static int estep_enqueue(phmrf_region *r, int estimate_type, bool want_post, bool want_pp = false,
-                         bool force_general = false) {
+                         bool overflow_redo = false) {
     if (!r) return PHMRF_E_INVALID;
     if (!r->have_logp || !r->have_labels) {
         set_error("phmrf_estep_stats: needs phmrf_emit_loglik and labels first");
@@ -875,7 +876,6 @@ static int estep_enqueue(phmrf_region *r, int estimate_type, bool want_post, boo
     a.partials = r->d_partials;
     a.stats_out = r->d_stats;
     a.flags = r->d_flags;
-    a.force_general = force_general ? 1 : 0;
     a.s_bound = ctx->beta * r->W * (estimate_type == 3 ? r->wmax : 1.0);
     a.nbr_g = nullptr;
     a.exp_beta = std::exp(ctx->beta);
@@ -886,7 +886,8 @@ static int estep_enqueue(phmrf_region *r, int estimate_type, bool want_post, boo
     a.grid_n2 = r->grid_n2;
     a.grid_rows = r->grid_rows;
     a.own_start_gid = r->own_start_gid;
-    if (ctx->potts && !force_general && !want_pp && r->W > 0 && std::fabs(a.s_bound) < 100.0) {
+    const bool bulk = !overflow_redo && estep_bulk_supported(a);
+    if (bulk) {
         // per-slot factors of the pipeline kernel: constant while beta and the weights are
         const int weighted = estimate_type == 3 ? 1 : 0;
         if (r->d_fwd) {
@@ -914,7 +915,7 @@ static int estep_enqueue(phmrf_region *r, int estimate_type, bool want_post, boo
         }
     }
     PHMRF_CUDA(cudaMemsetAsync(r->d_flags, 0, sizeof(int), r->stream));
-    return launch_estep(a, ctx->sm_count, r->stream);
+    return bulk ? launch_estep_bulk(a, ctx->sm_count, r->stream) : launch_estep(a, ctx->sm_count, r->stream);
 }
 
 int phmrf_estep_stats_async(phmrf_region *r, int estimate_type) { return estep_enqueue(r, estimate_type, false); }

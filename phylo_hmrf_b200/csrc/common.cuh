@@ -102,7 +102,7 @@ struct EstepArgs {
     double *partials;         // [sm_count][K*F + 3] per-CTA partial sums
     double *stats_out;        // [K*(1+D+D*D) + 3]
     int *flags;               // [1] device flag: bit 0 = the pipeline met an overflow, rerun on the general path
-    int force_general;        // skip the pipeline kernel
+    int64_t own_start_gid;    // region-global node id of the first owned node (implicit-grid form, below)
     double s_bound;           // upper bound of any neighbour weight sum: beta * W * max|w|
     const double *nbr_g;      // [W][ld] exp(beta * w) per slot (1 for an empty slot); pipeline kernel only
     double exp_beta;          // exp(beta)
@@ -113,15 +113,19 @@ struct EstepArgs {
     int grid_kind;            // 1 diagonal region (upper triangle), 0 rectangle, -1: explicit neighbour slots
     int grid_nn;              // 8 or 4
     int64_t grid_n2, grid_rows;
-    int64_t own_start_gid;    // region-global node id of the first owned node
 };
 // g[s][i] = exp(beta * (weighted ? w[s][i] : 1)) for occupied slots, 1 otherwise (kernels_b.cu)
 int launch_nbr_g(const int32_t *nbr_id, const double *nbr_w, double *nbr_g, int64_t count, double beta, int weighted,
                  cudaStream_t s);
+// The general kernel (kernels_b.cu): any V, any degree, any K; n == 0 zero-fills the statistics.
 int launch_estep(const EstepArgs &a, int sm_count, cudaStream_t s);
-// Warp-specialised bulk-copy pipeline (estep_bulk.cuh, kernels_b3*.cu), the fast path; *handled=false when the
-// shape is outside its range.
-int launch_estep_bulk(const EstepArgs &a, int sm_count, cudaStream_t s, bool *handled);
+// The one decision between the two phase-B kernels: true when the warp-specialised bulk-copy pipeline
+// (estep_bulk.cuh, kernels_b3*.cu) runs this E-step -- n > 0, no pp output, Potts V, 1..8 neighbour slots,
+// |s_bound| < 100, K <= 40 and a kernel shape that fits the registers and shared memory.  The caller then
+// fills nbr_g, or fwd_wg and grid_kind, and calls launch_estep_bulk, which returns PHMRF_E_UNSUPPORTED for
+// any other shape.  The redo after an overflow flag always takes the general kernel.
+bool estep_bulk_supported(const EstepArgs &a);
+int launch_estep_bulk(const EstepArgs &a, int sm_count, cudaStream_t s);
 // Fold per-block partials into stats_out (defined in kernels_b.cu).
 int launch_estep_finalize(const double *partials, int n_blocks, int K, int D, double *stats_out, cudaStream_t s);
 

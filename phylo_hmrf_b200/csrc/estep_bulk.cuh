@@ -24,28 +24,10 @@
 // (tools/swizzle_check.py), and a consumer addresses every operand of a step from
 // base ^ (step << 5) plus an immediate per 8-row tile.
 // exp() is a 2048-entry table (2^(j/2048), shared memory) times a quadratic: 6 FP64 instructions.
+// The variants measured and rejected for this kernel (neighbour data one tile ahead, sixteen producers, other
+// register budgets) are recorded in profiles/r2_history.md.
 #pragma once
 #include "estep_common.cuh"
-
-
-// experiment switches (tools/build_variant.sh): defaults are the shipped configuration
-#ifndef PHMRF_B3_PIPE_NBR
-#define PHMRF_B3_PIPE_NBR 0   // neighbour data loaded one tile ahead: measured slower (profiles/r2_history.md)
-#endif
-#ifndef PHMRF_B3_PROD_REGS
-#define PHMRF_B3_PROD_REGS 112  // P = 12, large accumulator tile: producer / consumer budgets
-#define PHMRF_B3_CONS_REGS 168  // (4*cons + 12*prod <= 2048)
-#endif
-#ifndef PHMRF_B3_PROD_REGS_SMALL
-#define PHMRF_B3_PROD_REGS_SMALL 120  // P = 12, small accumulator tile (NK8*NT <= 12)
-#define PHMRF_B3_CONS_REGS_SMALL 152
-#endif
-#ifndef PHMRF_B3_XEARLY
-#define PHMRF_B3_XEARLY 1     // feature loads issued before the neighbour factors are applied
-#endif
-#ifndef PHMRF_B3_P16
-#define PHMRF_B3_P16 0        // sixteen producer warps for small accumulator tiles: no faster than twelve (profiles/r2_history.md)
-#endif
 
 namespace phmrf {
 
@@ -184,28 +166,40 @@ __device__ __forceinline__ void write_y_rows(unsigned char *yb, const uint32_t (
     ((*reinterpret_cast<double *>(yb + colo[Fs & 7] + Fs * 256) = y_feature<D, Fs>(x, xs, inv)), ...);
 }
 
+// Shape of the kernel for D features and NK8 8-state tiles.  These functions are also what
+// estep_bulk_supported (kernels_b3.cu) evaluates at run time, so the launch chain and the host's choice of
+// kernel agree by construction.
+constexpr int kYSlots = 2;  // feature-row slots per consumer
+constexpr size_t kSmemMax = 227 * 1024;
+constexpr int bulk_nt(int D) { return (n_stat_features(D) + 7) / 8; }  // 8-feature tiles
+constexpr size_t bulk_smem_bytes(int D, int NK8, int P) {
+    return (size_t)P * (8 * NK8 * 256) + (size_t)kCons * kYSlots * (8 * bulk_nt(D) * 256) + kExpTab * 8 +
+           (3 * (size_t)P + kCons * kYSlots) * 8 + (size_t)P * 3 * 8 + 256;
+}
+// as many producer warps as shared memory and registers allow: the per-node work is latency bound
+constexpr int bulk_producers(int D, int NK8) {
+    return bulk_smem_bytes(D, NK8, 12) <= kSmemMax ? 12 : (bulk_smem_bytes(D, NK8, 8) <= kSmemMax ? 8 : 4);
+}
+// the consumer's NK8 x NT accumulator tiles (two doubles per lane each) fit its registers
+constexpr bool bulk_acc_fits(int D, int NK8) { return NK8 * bulk_nt(D) * 2 <= 64; }
+constexpr bool bulk_smem_fits(int D, int NK8) { return bulk_smem_bytes(D, NK8, bulk_producers(D, NK8)) <= kSmemMax; }
+
 template <int D, int NK8>
 struct BulkCfg {
     static constexpr int F = n_stat_features(D);
-    static constexpr int NT = (F + 7) / 8;
+    static constexpr int NT = bulk_nt(D);
     static constexpr int KP = 8 * NK8, FP = 8 * NT;
-    static constexpr int YS = 2;  // feature-row slots per consumer
+    static constexpr int YS = kYSlots;
     static constexpr int E_BYTES = KP * 256, Y_BYTES = FP * 256;
-    static constexpr size_t smem_bytes(int P) {
-        return (size_t)P * E_BYTES + (size_t)kCons * YS * Y_BYTES + kExpTab * 8 + (3 * (size_t)P + kCons * YS) * 8 + (size_t)P * 3 * 8 + 256;
-    }
-    // as many producer warps as shared memory and registers allow: the per-node work is latency
-    // bound.  Sixteen where the accumulator tile is small (every warp then fits 96 registers)
-    static constexpr int P = (PHMRF_B3_P16 && NK8 * NT <= 9 && D <= 6 && smem_bytes(16) <= 227 * 1024)
-                                 ? 16
-                                 : (smem_bytes(12) <= 227 * 1024 ? 12 : (smem_bytes(8) <= 227 * 1024 ? 8 : 4));
+    static constexpr int P = bulk_producers(D, NK8);
 };
 // register budgets after setmaxnreg (4 consumers + P producers share 2048 per lane column)
 template <int P, bool SMALL>
 struct RegBudget {
-    static constexpr int prod = P == 12 ? (SMALL ? PHMRF_B3_PROD_REGS_SMALL : PHMRF_B3_PROD_REGS) : (P == 8 ? 160 : 168);
-    static constexpr int cons = P == 12 ? (SMALL ? PHMRF_B3_CONS_REGS_SMALL : PHMRF_B3_CONS_REGS) : (P == 8 ? 184 : 168);
-    static constexpr bool adjust = P == 12 || P == 8;  // P = 4 and P = 16: every warp keeps the launch allocation
+    // P = 12: 112 / 168 for a large accumulator tile, 120 / 152 for a small one (NK8*NT <= 12)
+    static constexpr int prod = P == 12 ? (SMALL ? 120 : 112) : (P == 8 ? 160 : 168);
+    static constexpr int cons = P == 12 ? (SMALL ? 152 : 168) : (P == 8 ? 184 : 168);
+    static constexpr bool adjust = P == 12 || P == 8;  // P = 4: every warp keeps the launch allocation
 };
 
 // Row geometry of a dense region in the reference's node order (utility.py:2310-2317): node id -> (row x,
@@ -287,9 +281,7 @@ __global__ void __launch_bounds__(32 * (kCons + P), 1) estep_bulk_kernel(EstepAr
             const int64_t T0 = (int64_t)blockIdx.x * P + p;
             if (T0 < n_tiles) grid_locate(a.grid_kind, a.grid_n2, a.own_start_gid + T0 * kTile, gx, gc, gL);
         }
-        // ---- neighbour data of a tile, loaded one tile ahead (software pipeline): issued before the
-        // feature-row phase of the previous tile so that the global round trip is off the critical
-        // path; the registers below are dead between the soft-max of a tile and that point.
+        // ---- neighbour data of tile T, loaded at the top of tile T
         int li = 0;
         int lab[kFastSlots];
         double gw[kFastSlots];   // g_s = exp(beta*w_s) (precomputed, 1 if the slot is empty)
@@ -372,13 +364,12 @@ __global__ void __launch_bounds__(32 * (kCons + P), 1) estep_bulk_kernel(EstepAr
             }
             rmax = a.rowmax[i];
         };
-        if (PHMRF_B3_PIPE_NBR && (int64_t)blockIdx.x * P + p < n_tiles) load_neighbours((int64_t)blockIdx.x * P + p);
         for (int64_t T = (int64_t)blockIdx.x * P + p; T < n_tiles; T += tile_stride_g, ++j) {
             const int64_t i_raw = T * kTile + lane;
             const bool valid = i_raw < n;
             const int64_t i = valid ? i_raw : n - 1;
             {   // pull towards L2: this producer's next tile (log-likelihood, features) and the
-                // neighbour data of the tile after that (its register loads are issued during this tile)
+                // neighbour data of the tile after that
                 const int64_t T2 = T + tile_stride_g;
                 if (T2 < n_tiles) {
                     const int64_t i2 = T2 * kTile;
@@ -399,7 +390,7 @@ __global__ void __launch_bounds__(32 * (kCons + P), 1) estep_bulk_kernel(EstepAr
                     if (lane == 15) prefetch_l2(a.rowmax + i3);
                 }
             }
-            if (!PHMRF_B3_PIPE_NBR) load_neighbours(T);
+            load_neighbours(T);
             if constexpr (!GRID) {
 #pragma unroll
                 for (int s = 0; s < kFastSlots; ++s) lab[s] = jid[s] >= 0 ? a.labels[jid[s]] : -1;
@@ -498,13 +489,11 @@ __global__ void __launch_bounds__(32 * (kCons + P), 1) estep_bulk_kernel(EstepAr
             }
             // the node's features: in flight while the neighbour factors are applied
             double x[D];
-            if (PHMRF_B3_XEARLY) {
-                const double *px = a.X_soa + i;
+            const double *px = a.X_soa + i;
 #pragma unroll
-                for (int jx = 0; jx < D; ++jx) {
-                    x[jx] = *px;
-                    px += ld;
-                }
+            for (int jx = 0; jx < D; ++jx) {
+                x[jx] = *px;
+                px += ld;
             }
             // e_k *= g_s for every neighbour slot in turn (a label met twice is multiplied twice: the product)
 #pragma unroll
@@ -533,16 +522,6 @@ __global__ void __launch_bounds__(32 * (kCons + P), 1) estep_bulk_kernel(EstepAr
                         a.post_soa[q * ld + i] = *reinterpret_cast<double *>(eb + dyn_off(q)) * inv;
                 }
             }
-            // ---- the next tile's neighbour data: the loads fly during the feature-row phase
-            if (!PHMRF_B3_XEARLY) {
-                const double *px = a.X_soa + i;
-#pragma unroll
-                for (int jx = 0; jx < D; ++jx) {
-                    x[jx] = *px;
-                    px += ld;
-                }
-            }
-            if (PHMRF_B3_PIPE_NBR && T + tile_stride_g < n_tiles) load_neighbours(T + tile_stride_g);
             // ---- feature rows into the next Y slot of this producer's consumer (tile order)
             const int m = p / kCons + PPC * j;  // index among the consumer's tiles
             const int ys = m % YS;
@@ -663,11 +642,16 @@ __global__ void __launch_bounds__(32 * (kCons + P), 1) estep_bulk_kernel(EstepAr
     }
 }
 
+// a shape that estep_bulk_supported rejects reached the launcher: the caller's error, never a fall-back
+int bulk_unsupported(const EstepArgs &a) {
+    set_error("estep_bulk_kernel: no instantiation for n_features=" + std::to_string(a.D) +
+              ", n_states=" + std::to_string(a.K));
+    return PHMRF_E_UNSUPPORTED;
+}
+
 template <int D, int NK8, int P, int KR>
-int launch_bulk_pk(const EstepArgs &a, int sm_count, cudaStream_t s, bool *handled) {
-    using C = BulkCfg<D, NK8>;
-    size_t smem = C::smem_bytes(P);
-    if (smem > 227 * 1024) return PHMRF_OK;
+int launch_bulk_pk(const EstepArgs &a, int sm_count, cudaStream_t s) {
+    const size_t smem = bulk_smem_bytes(D, NK8, P);
     const int64_t n_tiles = (a.n + kTile - 1) / kTile;
     int64_t want = (n_tiles + P - 1) / P;
     const int grid = (int)(want < sm_count ? (want < 1 ? 1 : want) : sm_count);
@@ -676,73 +660,55 @@ int launch_bulk_pk(const EstepArgs &a, int sm_count, cudaStream_t s, bool *handl
     kern<<<grid, 32 * (kCons + P), smem, s>>>(a);
     count_launch();
     PHMRF_CUDA(cudaGetLastError());
-    *handled = true;
     return launch_estep_finalize(a.partials, grid, a.K, D, a.stats_out, s);
 }
 
 // KR: states of the last 8-state chunk that are evaluated (K's remainder rounded up to even); the
 // other rows of that chunk are padding and get zero weight without an exp()
 template <int D, int NK8, int P>
-int launch_bulk_p(const EstepArgs &a, int sm_count, cudaStream_t s, bool *handled) {
-    const int kr = (a.K - 8 * (NK8 - 1) + 1) & ~1;
-#ifdef PHMRF_B3_KR8
-    return launch_bulk_pk<D, NK8, P, 8>(a, sm_count, s, handled);
-#endif
-#ifdef PHMRF_B3_FAST_BUILD
-    if (kr == 6) return launch_bulk_pk<D, NK8, P, 6>(a, sm_count, s, handled);
-    if (kr == 4) return launch_bulk_pk<D, NK8, P, 4>(a, sm_count, s, handled);
-    return PHMRF_OK;
-#else
-    switch (kr) {
-        case 2: return launch_bulk_pk<D, NK8, P, 2>(a, sm_count, s, handled);
-        case 4: return launch_bulk_pk<D, NK8, P, 4>(a, sm_count, s, handled);
-        case 6: return launch_bulk_pk<D, NK8, P, 6>(a, sm_count, s, handled);
-        default: return launch_bulk_pk<D, NK8, P, 8>(a, sm_count, s, handled);
+int launch_bulk_p(const EstepArgs &a, int sm_count, cudaStream_t s) {
+    switch ((a.K - 8 * (NK8 - 1) + 1) & ~1) {
+        case 2: return launch_bulk_pk<D, NK8, P, 2>(a, sm_count, s);
+        case 4: return launch_bulk_pk<D, NK8, P, 4>(a, sm_count, s);
+        case 6: return launch_bulk_pk<D, NK8, P, 6>(a, sm_count, s);
+        default: return launch_bulk_pk<D, NK8, P, 8>(a, sm_count, s);
     }
-#endif
 }
 
 template <int D, int NK8>
-int launch_bulk(const EstepArgs &a, int sm_count, cudaStream_t s, bool *handled) {
-    using C = BulkCfg<D, NK8>;
-    if constexpr (NK8 * C::NT * 2 > 64) {
-        return PHMRF_OK;  // accumulator tiles would not fit the consumer's registers
+int launch_bulk(const EstepArgs &a, int sm_count, cudaStream_t s) {
+    if constexpr (!bulk_acc_fits(D, NK8) || !bulk_smem_fits(D, NK8)) {
+        return bulk_unsupported(a);
     } else {
-        return launch_bulk_p<D, NK8, C::P>(a, sm_count, s, handled);
+        return launch_bulk_p<D, NK8, BulkCfg<D, NK8>::P>(a, sm_count, s);
     }
 }
 
 template <int D>
-int launch_bulk_d(const EstepArgs &a, int sm_count, cudaStream_t s, bool *handled) {
-#ifdef PHMRF_B3_FAST_BUILD  // experiments: only the bench shapes
-    if constexpr (D == 9) { if ((a.K + 7) / 8 == 4) return launch_bulk<D, 4>(a, sm_count, s, handled); }
-    if constexpr (D == 5) { if ((a.K + 7) / 8 == 3) return launch_bulk<D, 3>(a, sm_count, s, handled); }
-    return PHMRF_OK;
-#else
+int launch_bulk_d(const EstepArgs &a, int sm_count, cudaStream_t s) {
     switch ((a.K + 7) / 8) {
-        case 1: return launch_bulk<D, 1>(a, sm_count, s, handled);
-        case 2: return launch_bulk<D, 2>(a, sm_count, s, handled);
-        case 3: return launch_bulk<D, 3>(a, sm_count, s, handled);
-        case 4: return launch_bulk<D, 4>(a, sm_count, s, handled);
-        case 5: return launch_bulk<D, 5>(a, sm_count, s, handled);
-        default: return PHMRF_OK;  // K > 40: general kernel
+        case 1: return launch_bulk<D, 1>(a, sm_count, s);
+        case 2: return launch_bulk<D, 2>(a, sm_count, s);
+        case 3: return launch_bulk<D, 3>(a, sm_count, s);
+        case 4: return launch_bulk<D, 4>(a, sm_count, s);
+        case 5: return launch_bulk<D, 5>(a, sm_count, s);
+        default: return bulk_unsupported(a);
     }
-#endif
 }
 
 }  // namespace
 
 // one translation unit per range of feature counts (kernels_b3.cu, kernels_b3_d58.cu, kernels_b3_d9c.cu):
 // the instantiations compile in parallel
-int PHMRF_B3_ENTRY(const EstepArgs &a, int sm_count, cudaStream_t s, bool *handled) {
+int PHMRF_B3_ENTRY(const EstepArgs &a, int sm_count, cudaStream_t s) {
     switch (a.D) {
 #define PHMRF_CASE(DD) \
     case DD:           \
-        return launch_bulk_d<DD>(a, sm_count, s, handled);
+        return launch_bulk_d<DD>(a, sm_count, s);
         PHMRF_CASE(PHMRF_B3_D0) PHMRF_CASE(PHMRF_B3_D0 + 1) PHMRF_CASE(PHMRF_B3_D0 + 2) PHMRF_CASE(PHMRF_B3_D0 + 3)
 #undef PHMRF_CASE
     }
-    return PHMRF_OK;
+    return bulk_unsupported(a);
 }
 
 }  // namespace phmrf

@@ -10,7 +10,7 @@ namespace phmrf {
 namespace estep {
 
 constexpr int kThreads = 256;
-constexpr int kFastSlots = 8;  // neighbour slots handled in registers by the fast node phase
+constexpr int kFastSlots = 8;  // neighbour slots kept in registers by the fast node phase
 
 __host__ __device__ constexpr int even_up(int v) { return (v + 1) & ~1; }
 // row strides (in doubles) are even (16-byte alignment of every row) with stride/2 odd, so

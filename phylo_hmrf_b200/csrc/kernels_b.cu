@@ -513,11 +513,6 @@ int launch_estep(const EstepArgs &a, int sm_count, cudaStream_t s) {
         PHMRF_CUDA(cudaMemsetAsync(a.stats_out, 0, sizeof(double) * (a.K * (1 + a.D + a.D * a.D) + 3), s));
         return PHMRF_OK;
     }
-    if (!a.force_general) {
-        bool handled = false;
-        int rc = launch_estep_bulk(a, sm_count, s, &handled);
-        if (rc != PHMRF_OK || handled) return rc;
-    }
     switch (a.D) {
 #define PHMRF_CASE(DD) \
     case DD:           \

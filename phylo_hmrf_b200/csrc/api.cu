@@ -2,9 +2,11 @@
 // kept on the host as the north star specifies), region upload / graph layout, and the
 // extern "C" entry points declared in include/phmrf.h.
 #include <atomic>
+#include <climits>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <vector>
 
@@ -45,54 +47,68 @@ struct phmrf_ctx {
     unsigned long long version = 0;
     std::vector<double> packed;  // K * model_stride(D)
     std::vector<double> V;       // K*K
-    double *d_model = nullptr;   // K * model_stride(D) packed factors
-    double *d_V = nullptr;
+    DevBuf<double> d_model;      // K * model_stride(D) packed factors
+    DevBuf<double> d_V;
 };
 
-struct phmrf_region {
-    phmrf_ctx *ctx = nullptr;
+// The stream a region runs on.  A base of phmrf_region, so that an owned stream is destroyed after the buffers.
+struct RegionStream {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
+    ~RegionStream() {
+        if (own_stream) cudaStreamDestroy(stream);
+        cudaGetLastError();  // teardown has no caller to report to
+    }
+};
+
+struct phmrf_region : RegionStream {
+    phmrf_ctx *ctx;
     int64_t n = 0, n_window = 0, own_offset = 0, ld = 0, E = 0;
     int W = 0;
     double wmax = 0.0;
-    double *d_X = nullptr;       // [D][ld]
-    double *d_logp = nullptr;    // tiled [ld/32][KP][32] (common.cuh lp_index)
-    double *d_rowmax = nullptr;  // [ld] max_k logp per node (written by the quantise kernel)
-    int32_t *d_unary = nullptr;  // [n][K]
-    int32_t *d_labels = nullptr; // [n_window]
-    int32_t *d_nbr_id = nullptr; // [W][ld]
-    double *d_nbr_w = nullptr;   // [W][ld]
-    double *d_nbr_g = nullptr;   // [W][ld] exp(beta*w), built on first use for (g_beta, g_weighted)
+    DevBuf<double> d_X;          // [D][ld]
+    DevBuf<double> d_logp;       // tiled [ld/32][KP][32] (common.cuh lp_index)
+    DevBuf<double> d_rowmax;     // [ld] max_k logp per node (written by the quantise kernel)
+    DevBuf<int32_t> d_unary;     // [n][K]
+    DevBuf<int32_t> d_labels;    // [n_window]
+    DevBuf<int32_t> d_nbr_id;    // [W][ld]
+    DevBuf<double> d_nbr_w;      // [W][ld]
+    DevBuf<double> d_nbr_g;      // [W][ld] exp(beta*w), built on first use for (g_beta, g_weighted)
     // implicit-grid form (phmrf_region_create_grid): forward-edge {w, exp(beta*w)} per window node
-    double2 *d_fwd = nullptr;    // [4][ldw]
+    DevBuf<double2> d_fwd;       // [4][ldw]
     int64_t ldw = 0, own_start_gid = 0, grid_n2 = 0, grid_rows = 0;
     int grid_kind = -1, grid_nn = 0;
     double fwd_beta = 0.0;
     int fwd_weighted = -1;
     double g_beta = 0.0;
     int g_weighted = -1;
-    double *d_edge_w = nullptr;  // [E]
-    int32_t *d_edge_wi = nullptr;
-    long long *d_edge_ids = nullptr;  // [E,2] window-local, only for regions built by phmrf_region_create_grid
-    unsigned long long *d_absmax = nullptr;  // [1] bits, [1] boundary counter
-    double *d_dwf = nullptr;                 // [2] dwf, absmax
-    long long *d_blist = nullptr;
+    DevBuf<double> d_edge_w;     // [E]
+    DevBuf<int32_t> d_edge_wi;
+    DevBuf<long long> d_edge_ids;          // [E,2] window-local, only for regions built by phmrf_region_create_grid
+    DevBuf<unsigned long long> d_absmax;   // [1] bits, [1] boundary counter
+    DevBuf<double> d_dwf;                  // [2] dwf, absmax
+    DevBuf<long long> d_blist;
     long long bcap = 0;
-    double *d_partials = nullptr;
-    double *d_stats = nullptr;
-    int *d_flags = nullptr;
-    long long *d_badlabel = nullptr;  // [1] first out-of-range label index, -1 if none
-    double *d_scratch = nullptr;  // [K][ld] posteriors / AoS staging, allocated on demand
+    DevBuf<double> d_partials;
+    DevBuf<double> d_stats;
+    DevBuf<int> d_flags;
+    DevBuf<long long> d_badlabel;  // [1] first out-of-range label index, -1 if none
+    DevBuf<double> d_scratch;      // [K][ld] posteriors / AoS staging, allocated on demand
     int64_t scratch_elems = 0;
     bool have_logp = false, have_unary = false, have_labels = false, have_rowmax = false;
     bool edges_sorted = true;   // edge list sorted by (id1, id2): the device cut numbers the edges from the slots
-    SwapScratch *cut = nullptr; // device graph cut, allocated at the first phmrf_region_graph_cut
+    std::unique_ptr<SwapScratch> cut;  // device graph cut, allocated at the first phmrf_region_graph_cut
     int64_t bytes = 0;
     // small results (statistics, flags, dwf, counters) come back through a host-mapped buffer that a
     // kernel writes (launch_publish), not through the copy engines
-    unsigned long long *h_small = nullptr;  // host view
-    unsigned long long *d_small = nullptr;  // device view of the same memory
+    MappedBuf small;
+
+    explicit phmrf_region(phmrf_ctx *c) : ctx(c) {}
+    // The regions of one process live on different GPUs: free on the region's own, after its queued work.
+    ~phmrf_region() {
+        cudaSetDevice(ctx->device);
+        if (stream) cudaStreamSynchronize(stream);
+    }
 };
 
 // word offsets inside the mapped buffer
@@ -105,11 +121,15 @@ int set_device(const phmrf_ctx *ctx) {
     return PHMRF_OK;
 }
 
-template <typename T>
-int dev_alloc(phmrf_region *r, T **p, int64_t count) {
-    if (count <= 0) count = 1;
-    PHMRF_CUDA(cudaMalloc((void **)p, sizeof(T) * (size_t)count));
-    r->bytes += (int64_t)sizeof(T) * count;
+// Makes `device` current; PHMRF_E_CUDA when there is no such device, or it is not below `limit`.
+int use_device(int device, const char *who, int limit = INT_MAX) {
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || device < 0 || device >= count || device >= limit) {
+        cudaGetLastError();
+        set_error(std::string(who) + ": no such CUDA device (this library has no CPU fallback)");
+        return PHMRF_E_CUDA;
+    }
+    PHMRF_CUDA(cudaSetDevice(device));
     return PHMRF_OK;
 }
 
@@ -131,31 +151,89 @@ bool cholesky_lower(const double *A, int d, double shift, std::vector<double> &L
     return true;
 }
 
-int alloc_small(phmrf_region *r) {
-    const size_t words = (size_t)kSmStats + (size_t)phmrf_stats_len(r->ctx);
-    void *h = nullptr, *d = nullptr;
-    PHMRF_CUDA(cudaHostAlloc(&h, words * sizeof(unsigned long long), cudaHostAllocMapped | cudaHostAllocPortable));
-    if (cudaHostGetDevicePointer(&d, h, 0) != cudaSuccess) {
-        cudaError_t e = cudaGetLastError();
-        cudaFreeHost(h);
-        return cuda_fail(e, "cudaHostGetDevicePointer", __FILE__, __LINE__);
+int ensure_scratch(phmrf_region *r, int64_t elems) {
+    if (r->scratch_elems >= elems) return PHMRF_OK;
+    r->bytes -= r->scratch_elems * (int64_t)sizeof(double);
+    r->scratch_elems = 0;
+    int rc = r->d_scratch.alloc(elems, &r->bytes);
+    if (rc == PHMRF_OK) r->scratch_elems = elems;
+    return rc;
+}
+
+// A region on the caller's stream, or on a non-blocking stream of its own.  The region's buffers come after
+// (region_alloc): a grid region counts its edges on this stream before they can be sized.
+int region_open(phmrf_ctx *ctx, void *stream, std::unique_ptr<phmrf_region> &r) {
+    r.reset(new phmrf_region(ctx));
+    if (stream) {
+        r->stream = (cudaStream_t)stream;
+        return PHMRF_OK;
     }
-    r->h_small = static_cast<unsigned long long *>(h);
-    r->d_small = static_cast<unsigned long long *>(d);
+    cudaStream_t s = nullptr;
+    if (cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking) != cudaSuccess)
+        return cuda_fail(cudaGetLastError(), "cudaStreamCreate", __FILE__, __LINE__);
+    r->stream = s;
+    r->own_stream = true;
     return PHMRF_OK;
 }
 
-int ensure_scratch(phmrf_region *r, int64_t elems) {
-    if (r->scratch_elems >= elems) return PHMRF_OK;
-    if (r->d_scratch) {
-        cudaFree(r->d_scratch);
-        r->bytes -= r->scratch_elems * (int64_t)sizeof(double);
-        r->d_scratch = nullptr;
-        r->scratch_elems = 0;
-    }
-    int rc = dev_alloc(r, &r->d_scratch, elems);
-    if (rc == PHMRF_OK) r->scratch_elems = elems;
-    return rc;
+// Every buffer both region kinds share, counted in r->bytes; then X, rowmax and the log-likelihood (with its
+// padding rows, common.cuh logp_rows) are cleared on the region's stream.
+int region_alloc(phmrf_region *r, int64_t n_own, int64_t n_window, int64_t own_offset, int W, int64_t E) {
+    const phmrf_ctx *ctx = r->ctx;
+    const int K = ctx->K, D = ctx->D;
+    r->n = n_own;
+    r->n_window = n_window;
+    r->own_offset = own_offset;
+    r->W = W;
+    r->E = E;
+    r->ld = round_up(n_own > 0 ? n_own : 1, 64);
+    r->bcap = 1 << 20;
+    const int64_t ld = r->ld, stats_len = phmrf_stats_len(ctx);
+    int64_t *b = &r->bytes;
+    int rc;
+    if ((rc = r->d_X.alloc((int64_t)D * ld, b)) || (rc = r->d_logp.alloc((int64_t)logp_rows(K) * ld, b)) ||
+        (rc = r->d_rowmax.alloc(ld, b)) || (rc = r->d_unary.alloc(n_own * K, b)) ||
+        (rc = r->d_labels.alloc(n_window, b)) || (rc = r->d_nbr_id.alloc((int64_t)W * ld, b)) ||
+        (rc = r->d_nbr_w.alloc((int64_t)W * ld, b)) || (rc = r->d_edge_w.alloc(E, b)) ||
+        (rc = r->d_edge_wi.alloc(E, b)) || (rc = r->d_absmax.alloc(2, b)) || (rc = r->d_dwf.alloc(2, b)) ||
+        (rc = r->d_blist.alloc(r->bcap, b)) ||
+        (rc = r->d_partials.alloc((int64_t)ctx->sm_count * ((int64_t)K * n_stat_features(D) + 3), b)) ||
+        (rc = r->d_stats.alloc(stats_len, b)) || (rc = r->d_flags.alloc(1, b)) || (rc = r->d_badlabel.alloc(1, b)) ||
+        (rc = r->small.alloc((size_t)(kSmStats + stats_len))))
+        return rc;
+    if (n_own == 0) return PHMRF_OK;
+    if (cudaMemsetAsync(r->d_X, 0, sizeof(double) * D * ld, r->stream) != cudaSuccess ||
+        cudaMemsetAsync(r->d_rowmax, 0, sizeof(double) * ld, r->stream) != cudaSuccess)
+        return cuda_fail(cudaGetLastError(), "memset X", __FILE__, __LINE__);
+    return launch_logp_init(r->d_logp, ld, K, r->stream);
+}
+
+// V as the graph cut takes it: numpy's (V * _SMOOTH_COST_PRECISION).astype(intc), K*K values
+void smooth_costs_i32(const phmrf_ctx *ctx, int32_t *V_i32) {
+    for (int i = 0; i < ctx->K * ctx->K; ++i) V_i32[i] = (int32_t)(ctx->V[i] * ctx->sprec);
+}
+
+// Uploads n labels and checks their range on the device (a host loop over 4e7 labels costs more than the
+// copy): *first_bad is the index of the first label outside [0, K), or -1.
+int upload_labels(phmrf_region *r, const int32_t *labels, int64_t n, long long *first_bad) {
+    PHMRF_CUDA(cudaMemcpyAsync(r->d_labels, labels, sizeof(int32_t) * n, cudaMemcpyHostToDevice, r->stream));
+    int rc;
+    if ((rc = launch_check_labels(r->d_labels, n, r->ctx->K, r->d_badlabel, r->stream)) != PHMRF_OK) return rc;
+    if ((rc = launch_publish(r->small.dev + kSmBadLabel, r->d_badlabel, 1, false, r->stream)) != PHMRF_OK) return rc;
+    PHMRF_CUDA(cudaStreamSynchronize(r->stream));
+    *first_bad = (long long)r->small.host[kSmBadLabel];
+    return PHMRF_OK;
+}
+
+// Enqueues the download of the [K][ld] array at the start of the scratch as [n,K] rows, staged behind it.
+int enqueue_rows_download(phmrf_region *r, double *out) {
+    if (r->n == 0) return PHMRF_OK;
+    const int K = r->ctx->K;
+    double *aos = r->d_scratch + (int64_t)K * r->ld;
+    int rc = launch_soa_to_aos(r->d_scratch, aos, r->n, K, r->ld, r->stream);
+    if (rc) return rc;
+    PHMRF_CUDA(cudaMemcpyAsync(out, aos, sizeof(double) * r->n * K, cudaMemcpyDeviceToHost, r->stream));
+    return PHMRF_OK;
 }
 
 }  // namespace
@@ -187,39 +265,25 @@ int phmrf_ctx_create(int device, int n_states, int n_features, phmrf_ctx **out) 
         set_error("phmrf_ctx_create: need n_states>=1 and 1<=n_features<=12");
         return n_features > kMaxFeatures ? PHMRF_E_UNSUPPORTED : PHMRF_E_INVALID;
     }
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess || device < 0 || device >= count || device >= 64) {
-        cudaGetLastError();
-        set_error("phmrf_ctx_create: no such CUDA device (this library has no CPU fallback)");
-        return PHMRF_E_CUDA;
-    }
-    PHMRF_CUDA(cudaSetDevice(device));
-    phmrf_ctx *ctx = new phmrf_ctx();
+    // below 64: g_h2d_turn and g_d2h_turn hold one transfer turn per device
+    int rc = use_device(device, "phmrf_ctx_create", 64);
+    if (rc) return rc;
+    std::unique_ptr<phmrf_ctx> ctx(new phmrf_ctx());
     ctx->device = device;
     ctx->K = n_states;
     ctx->D = n_features;
-    if (cudaDeviceGetAttribute(&ctx->sm_count, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) {
-        delete ctx;
+    if (cudaDeviceGetAttribute(&ctx->sm_count, cudaDevAttrMultiProcessorCount, device) != cudaSuccess)
         return cuda_fail(cudaGetLastError(), "cudaDeviceGetAttribute", __FILE__, __LINE__);
-    }
-    const size_t md = (size_t)n_states * model_stride(n_features);
-    if (cudaMalloc((void **)&ctx->d_model, sizeof(double) * md) != cudaSuccess ||
-        cudaMalloc((void **)&ctx->d_V, sizeof(double) * n_states * n_states) != cudaSuccess) {
-        cudaError_t err = cudaGetLastError();
-        if (ctx->d_model) cudaFree(ctx->d_model);
-        delete ctx;
-        return cuda_fail(err, "cudaMalloc(model)", __FILE__, __LINE__);
-    }
-    *out = ctx;
+    if ((rc = ctx->d_model.alloc((int64_t)n_states * model_stride(n_features))) ||
+        (rc = ctx->d_V.alloc((int64_t)n_states * n_states)))
+        return rc;
+    *out = ctx.release();
     return PHMRF_OK;
 }
 
 int phmrf_ctx_destroy(phmrf_ctx *ctx) {
     if (!ctx) return PHMRF_OK;
     cudaSetDevice(ctx->device);
-    cudaFree(ctx->d_model);
-    cudaFree(ctx->d_V);
     delete ctx;
     return PHMRF_OK;
 }
@@ -330,7 +394,7 @@ int phmrf_region_create(phmrf_ctx *ctx, const double *X, int64_t n_own, int64_t 
     }
     int rc = set_device(ctx);
     if (rc) return rc;
-    const int K = ctx->K, D = ctx->D;
+    const int D = ctx->D;
     // ---- graph layout on the host: per owned node, its neighbours in ascending edge order
     std::vector<int> deg((size_t)n_own, 0);
     double wmax = 0.0;
@@ -351,64 +415,19 @@ int phmrf_region_create(phmrf_ctx *ctx, const double *X, int64_t n_own, int64_t 
     int W = 0;
     for (int64_t i = 0; i < n_own; ++i) W = deg[i] > W ? deg[i] : W;
 
-    phmrf_region *r = new phmrf_region();
-    r->ctx = ctx;
-    r->n = n_own;
-    r->n_window = n_window;
-    r->own_offset = own_offset;
-    r->E = n_edges;
-    r->W = W;
+    std::unique_ptr<phmrf_region> r;
+    if ((rc = region_open(ctx, stream, r)) || (rc = region_alloc(r.get(), n_own, n_window, own_offset, W, n_edges)))
+        return rc;
     r->wmax = wmax;
     r->edges_sorted = sorted;
-    r->ld = round_up(n_own > 0 ? n_own : 1, 64);
-    if (stream) {
-        r->stream = (cudaStream_t)stream;
-    } else {
-        if (cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking) != cudaSuccess) {
-            delete r;
-            return cuda_fail(cudaGetLastError(), "cudaStreamCreate", __FILE__, __LINE__);
-        }
-        r->own_stream = true;
-    }
     const int64_t ld = r->ld;
-    const int F = n_stat_features(D);
-#define TRY(x)                     \
-    if ((rc = (x)) != PHMRF_OK) {  \
-        phmrf_region_destroy(r);   \
-        return rc;                 \
-    }
-    TRY(dev_alloc(r, &r->d_X, (int64_t)D * ld));
-    TRY(dev_alloc(r, &r->d_logp, (int64_t)logp_rows(K) * ld));
-    TRY(dev_alloc(r, &r->d_rowmax, ld));
-    TRY(dev_alloc(r, &r->d_unary, n_own * K));
-    TRY(dev_alloc(r, &r->d_labels, n_window));
-    TRY(dev_alloc(r, &r->d_nbr_id, (int64_t)W * ld));
-    TRY(dev_alloc(r, &r->d_nbr_w, (int64_t)W * ld));
-    TRY(dev_alloc(r, &r->d_edge_w, n_edges));
-    TRY(dev_alloc(r, &r->d_edge_wi, n_edges));
-    TRY(dev_alloc(r, &r->d_absmax, 2));
-    TRY(dev_alloc(r, &r->d_dwf, 2));
-    r->bcap = 1 << 20;
-    TRY(dev_alloc(r, &r->d_blist, r->bcap));
-    TRY(dev_alloc(r, &r->d_partials, (int64_t)ctx->sm_count * ((int64_t)K * F + 3)));
-    TRY(dev_alloc(r, &r->d_stats, phmrf_stats_len(ctx)));
-    TRY(dev_alloc(r, &r->d_flags, 1));
-    TRY(dev_alloc(r, &r->d_badlabel, 1));
-    TRY(alloc_small(r));
-
     // X: upload row-major, transpose on the device into the feature-major layout
     if (n_own > 0) {
-        TRY(ensure_scratch(r, n_own * D));
-        if (cudaMemsetAsync(r->d_X, 0, sizeof(double) * D * ld, r->stream) != cudaSuccess ||
-            cudaMemsetAsync(r->d_rowmax, 0, sizeof(double) * ld, r->stream) != cudaSuccess ||
-            launch_logp_init(r->d_logp, ld, K, r->stream) != PHMRF_OK ||
-            cudaMemcpyAsync(r->d_scratch, X, sizeof(double) * n_own * D, cudaMemcpyHostToDevice, r->stream) !=
-                cudaSuccess) {
-            cudaError_t err = cudaGetLastError();
-            phmrf_region_destroy(r);
-            return cuda_fail(err, "upload X", __FILE__, __LINE__);
-        }
-        TRY(launch_aos_to_soa(r->d_scratch, r->d_X, n_own, D, ld, r->stream));
+        if ((rc = ensure_scratch(r.get(), n_own * D)) != PHMRF_OK) return rc;
+        if (cudaMemcpyAsync(r->d_scratch, X, sizeof(double) * n_own * D, cudaMemcpyHostToDevice, r->stream) !=
+            cudaSuccess)
+            return cuda_fail(cudaGetLastError(), "upload X", __FILE__, __LINE__);
+        if ((rc = launch_aos_to_soa(r->d_scratch, r->d_X, n_own, D, ld, r->stream)) != PHMRF_OK) return rc;
     }
     if (W > 0) {
         std::vector<int32_t> nid((size_t)W * ld, -1);
@@ -430,25 +449,15 @@ int phmrf_region_create(phmrf_ctx *ctx, const double *X, int64_t n_own, int64_t 
             }
         }
         if (cudaMemcpy(r->d_nbr_id, nid.data(), sizeof(int32_t) * nid.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
-            cudaMemcpy(r->d_nbr_w, nw.data(), sizeof(double) * nw.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
-            cudaError_t err = cudaGetLastError();
-            phmrf_region_destroy(r);
-            return cuda_fail(err, "upload graph", __FILE__, __LINE__);
-        }
+            cudaMemcpy(r->d_nbr_w, nw.data(), sizeof(double) * nw.size(), cudaMemcpyHostToDevice) != cudaSuccess)
+            return cuda_fail(cudaGetLastError(), "upload graph", __FILE__, __LINE__);
     }
     if (n_edges > 0 &&
-        cudaMemcpy(r->d_edge_w, edge_w, sizeof(double) * n_edges, cudaMemcpyHostToDevice) != cudaSuccess) {
-        cudaError_t err = cudaGetLastError();
-        phmrf_region_destroy(r);
-        return cuda_fail(err, "upload edge weights", __FILE__, __LINE__);
-    }
-    if (cudaStreamSynchronize(r->stream) != cudaSuccess) {
-        cudaError_t err = cudaGetLastError();
-        phmrf_region_destroy(r);
-        return cuda_fail(err, "region upload", __FILE__, __LINE__);
-    }
-#undef TRY
-    *out = r;
+        cudaMemcpy(r->d_edge_w, edge_w, sizeof(double) * n_edges, cudaMemcpyHostToDevice) != cudaSuccess)
+        return cuda_fail(cudaGetLastError(), "upload edge weights", __FILE__, __LINE__);
+    if (cudaStreamSynchronize(r->stream) != cudaSuccess)
+        return cuda_fail(cudaGetLastError(), "region upload", __FILE__, __LINE__);
+    *out = r.release();
     return PHMRF_OK;
 }
 
@@ -462,7 +471,7 @@ int phmrf_region_create_grid(phmrf_ctx *ctx, const double *X_window, int kind, i
     }
     int rc = set_device(ctx);
     if (rc) return rc;
-    const int K = ctx->K, D = ctx->D;
+    const int D = ctx->D;
     const int64_t h0 = row0 > 0 ? row0 - 1 : 0, h1 = row1 < rows ? row1 + 1 : rows;
     const int64_t win_start = grid_row_start(kind, n1, n2, h0), win_end = grid_row_start(kind, n1, n2, h1);
     const int64_t own_start = grid_row_start(kind, n1, n2, row0), own_end = grid_row_start(kind, n1, n2, row1);
@@ -471,71 +480,19 @@ int phmrf_region_create_grid(phmrf_ctx *ctx, const double *X_window, int kind, i
         set_error("phmrf_region_create_grid: window too large for 32-bit neighbour ids");
         return PHMRF_E_INVALID;
     }
-    phmrf_region *r = new phmrf_region();
-    r->ctx = ctx;
-    r->n = n_own;
-    r->n_window = n_window;
-    r->own_offset = own_start - win_start;
-    r->W = num_neighbor;
-    r->ld = round_up(n_own > 0 ? n_own : 1, 64);
-    if (stream) {
-        r->stream = (cudaStream_t)stream;
-    } else {
-        if (cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking) != cudaSuccess) {
-            delete r;
-            return cuda_fail(cudaGetLastError(), "cudaStreamCreate", __FILE__, __LINE__);
-        }
-        r->own_stream = true;
-    }
-    const int64_t ld = r->ld;
-    const int F = n_stat_features(D);
-    double *dXw = nullptr;
-#define TRY(x)                     \
-    if ((rc = (x)) != PHMRF_OK) {  \
-        cudaFree(dXw);             \
-        phmrf_region_destroy(r);   \
-        return rc;                 \
-    }
-    if (cudaMalloc((void **)&dXw, sizeof(double) * n_window * D) != cudaSuccess ||
-        cudaMemcpyAsync(dXw, X_window, sizeof(double) * n_window * D, cudaMemcpyHostToDevice, r->stream) !=
-            cudaSuccess) {
-        cudaError_t err = cudaGetLastError();
-        cudaFree(dXw);
-        phmrf_region_destroy(r);
-        return cuda_fail(err, "upload X window", __FILE__, __LINE__);
-    }
-    long long n_edges = 0;
-    TRY(dev_alloc(r, &r->d_absmax, 2));
-    TRY(launch_band_graph(dXw, kind, n1, n2, num_neighbor, D, win_start, own_start, own_end, n_window, beta1, ld,
-                          nullptr, nullptr, nullptr, nullptr, &n_edges, nullptr, r->stream));
-    r->E = n_edges;
-    TRY(dev_alloc(r, &r->d_X, (int64_t)D * ld));
-    TRY(dev_alloc(r, &r->d_logp, (int64_t)logp_rows(K) * ld));
-    TRY(dev_alloc(r, &r->d_rowmax, ld));
-    TRY(dev_alloc(r, &r->d_unary, n_own * K));
-    TRY(dev_alloc(r, &r->d_labels, n_window));
-    TRY(dev_alloc(r, &r->d_nbr_id, (int64_t)r->W * ld));
-    TRY(dev_alloc(r, &r->d_nbr_w, (int64_t)r->W * ld));
-    TRY(dev_alloc(r, &r->d_edge_w, n_edges));
-    TRY(dev_alloc(r, &r->d_edge_wi, n_edges));
-    TRY(dev_alloc(r, &r->d_edge_ids, 2 * n_edges));
-    TRY(dev_alloc(r, &r->d_dwf, 2));
-    r->bcap = 1 << 20;
-    TRY(dev_alloc(r, &r->d_blist, r->bcap));
-    TRY(dev_alloc(r, &r->d_partials, (int64_t)ctx->sm_count * ((int64_t)K * F + 3)));
-    TRY(dev_alloc(r, &r->d_stats, phmrf_stats_len(ctx)));
-    TRY(dev_alloc(r, &r->d_flags, 1));
-    TRY(dev_alloc(r, &r->d_badlabel, 1));
-    TRY(alloc_small(r));
-    if (cudaMemsetAsync(r->d_X, 0, sizeof(double) * D * ld, r->stream) != cudaSuccess ||
-        cudaMemsetAsync(r->d_rowmax, 0, sizeof(double) * ld, r->stream) != cudaSuccess ||
-        launch_logp_init(r->d_logp, ld, K, r->stream) != PHMRF_OK) {
-        cudaError_t err = cudaGetLastError();
-        cudaFree(dXw);
-        phmrf_region_destroy(r);
-        return cuda_fail(err, "memset X", __FILE__, __LINE__);
-    }
-    TRY(launch_aos_to_soa(dXw + r->own_offset * D, r->d_X, n_own, D, ld, r->stream));
+    std::unique_ptr<phmrf_region> r;
+    if ((rc = region_open(ctx, stream, r)) != PHMRF_OK) return rc;
+    DevBuf<double> dXw;  // the window's features [n_window, D], only while the region is built
+    if ((rc = dXw.alloc(n_window * D)) != PHMRF_OK) return rc;
+    if (cudaMemcpyAsync(dXw, X_window, sizeof(double) * n_window * D, cudaMemcpyHostToDevice, r->stream) != cudaSuccess)
+        return cuda_fail(cudaGetLastError(), "upload X window", __FILE__, __LINE__);
+    long long n_edges = 0;  // the counting call: the edge count sizes the edge buffers
+    if ((rc = launch_band_graph(dXw, kind, n1, n2, num_neighbor, D, win_start, own_start, own_end, n_window, beta1, 0,
+                                nullptr, nullptr, nullptr, nullptr, &n_edges, nullptr, r->stream)) ||
+        (rc = region_alloc(r.get(), n_own, n_window, own_start - win_start, num_neighbor, n_edges)) ||
+        (rc = r->d_edge_ids.alloc(2 * n_edges, &r->bytes)))
+        return rc;
+    if ((rc = launch_aos_to_soa(dXw + r->own_offset * D, r->d_X, n_own, D, r->ld, r->stream)) != PHMRF_OK) return rc;
     // implicit-grid form of phase B: one {w, g} pair per forward edge of every window node up to the last owned one
     r->grid_kind = kind;
     r->grid_nn = num_neighbor;
@@ -543,29 +500,22 @@ int phmrf_region_create_grid(phmrf_ctx *ctx, const double *X_window, int kind, i
     r->grid_rows = rows;
     r->own_start_gid = own_start;
     r->ldw = round_up(r->own_offset + n_own > 0 ? r->own_offset + n_own : 1, 64);
-    TRY(dev_alloc(r, &r->d_fwd, 4 * r->ldw));
-    if (cudaMemsetAsync(r->d_fwd, 0, sizeof(double2) * 4 * r->ldw, r->stream) != cudaSuccess) {  // incl. the row padding
-        cudaError_t err = cudaGetLastError();
-        cudaFree(dXw);
-        phmrf_region_destroy(r);
-        return cuda_fail(err, "memset forward weights", __FILE__, __LINE__);
-    }
-    TRY(launch_band_fwd(dXw, kind, n1, n2, num_neighbor, D, win_start, r->own_offset + n_own, beta1, r->ldw, r->d_fwd,
-                        r->stream));
+    if ((rc = r->d_fwd.alloc(4 * r->ldw, &r->bytes)) != PHMRF_OK) return rc;
+    if (cudaMemsetAsync(r->d_fwd, 0, sizeof(double2) * 4 * r->ldw, r->stream) != cudaSuccess)  // incl. the row padding
+        return cuda_fail(cudaGetLastError(), "memset forward weights", __FILE__, __LINE__);
+    if ((rc = launch_band_fwd(dXw, kind, n1, n2, num_neighbor, D, win_start, r->own_offset + n_own, beta1, r->ldw,
+                              r->d_fwd, r->stream)) != PHMRF_OK)
+        return rc;
     // max|w| lands in d_absmax[1] (free until the first quantise resets it as the boundary counter)
-    TRY(launch_band_graph(dXw, kind, n1, n2, num_neighbor, D, win_start, own_start, own_end, n_window, beta1, ld,
-                          r->d_nbr_id, r->d_nbr_w, r->d_edge_ids, r->d_edge_w, &n_edges, r->d_absmax + 1, r->stream));
+    if ((rc = launch_band_graph(dXw, kind, n1, n2, num_neighbor, D, win_start, own_start, own_end, n_window, beta1,
+                                r->ld, r->d_nbr_id, r->d_nbr_w, r->d_edge_ids, r->d_edge_w, &n_edges, r->d_absmax + 1,
+                                r->stream)) != PHMRF_OK)
+        return rc;
     unsigned long long wbits = 0;
-    if (cudaMemcpy(&wbits, r->d_absmax + 1, sizeof(wbits), cudaMemcpyDeviceToHost) != cudaSuccess) {
-        cudaError_t err = cudaGetLastError();
-        cudaFree(dXw);
-        phmrf_region_destroy(r);
-        return cuda_fail(err, "read max|w|", __FILE__, __LINE__);
-    }
+    if (cudaMemcpy(&wbits, r->d_absmax + 1, sizeof(wbits), cudaMemcpyDeviceToHost) != cudaSuccess)
+        return cuda_fail(cudaGetLastError(), "read max|w|", __FILE__, __LINE__);
     std::memcpy(&r->wmax, &wbits, sizeof(double));
-#undef TRY
-    cudaFree(dXw);
-    *out = r;
+    *out = r.release();
     return PHMRF_OK;
 }
 
@@ -634,36 +584,6 @@ int phmrf_region_update_X(phmrf_region *r, const double *X) {
 }
 
 int phmrf_region_destroy(phmrf_region *r) {
-    if (!r) return PHMRF_OK;
-    cudaSetDevice(r->ctx->device);
-    if (r->stream) cudaStreamSynchronize(r->stream);
-    cudaFree(r->d_X);
-    cudaFree(r->d_logp);
-    cudaFree(r->d_rowmax);
-    cudaFree(r->d_unary);
-    cudaFree(r->d_labels);
-    cudaFree(r->d_nbr_id);
-    cudaFree(r->d_nbr_w);
-    cudaFree(r->d_nbr_g);
-    cudaFree(r->d_fwd);
-    cudaFree(r->d_edge_w);
-    cudaFree(r->d_edge_wi);
-    cudaFree(r->d_edge_ids);
-    cudaFree(r->d_absmax);
-    cudaFree(r->d_dwf);
-    cudaFree(r->d_blist);
-    cudaFree(r->d_partials);
-    cudaFree(r->d_stats);
-    cudaFree(r->d_flags);
-    cudaFree(r->d_badlabel);
-    cudaFree(r->d_scratch);
-    if (r->cut) {
-        swap_scratch_free(*r->cut);
-        delete r->cut;
-    }
-    if (r->h_small) cudaFreeHost(r->h_small);
-    if (r->own_stream) cudaStreamDestroy(r->stream);
-    cudaGetLastError();
     delete r;
     return PHMRF_OK;
 }
@@ -680,8 +600,8 @@ int64_t phmrf_stats_len(const phmrf_ctx *ctx) {
     return ctx ? (int64_t)ctx->K * (1 + ctx->D + ctx->D * ctx->D) + 3 : 0;
 }
 
-void *phmrf_stats_device_ptr(phmrf_region *r) { return r ? (void *)r->d_stats : nullptr; }
-void *phmrf_absmax_device_ptr(phmrf_region *r) { return r ? (void *)r->d_absmax : nullptr; }
+void *phmrf_stats_device_ptr(phmrf_region *r) { return r ? (void *)r->d_stats.get() : nullptr; }
+void *phmrf_absmax_device_ptr(phmrf_region *r) { return r ? (void *)r->d_absmax.get() : nullptr; }
 double phmrf_region_weight_max(const phmrf_region *r) { return r ? r->wmax : 0.0; }
 int phmrf_region_set_weight_max(phmrf_region *r, double wmax) {
     if (!r || !(wmax >= 0.0)) return PHMRF_E_INVALID;
@@ -713,9 +633,9 @@ int phmrf_emit_loglik(phmrf_region *r, double *absmax_out) {
     int rc = phmrf_emit_loglik_async(r);
     if (rc) return rc;
     if (absmax_out) {
-        if ((rc = launch_publish(r->d_small + kSmAbsmax, r->d_absmax, 1, false, r->stream)) != PHMRF_OK) return rc;
+        if ((rc = launch_publish(r->small.dev + kSmAbsmax, r->d_absmax, 1, false, r->stream)) != PHMRF_OK) return rc;
         PHMRF_CUDA(cudaStreamSynchronize(r->stream));
-        std::memcpy(absmax_out, r->h_small + kSmAbsmax, sizeof(double));
+        std::memcpy(absmax_out, r->small.host + kSmAbsmax, sizeof(double));
     }
     return PHMRF_OK;
 }
@@ -751,7 +671,7 @@ int phmrf_quantise_async(phmrf_region *r, double dwf_in, double tol) {
     // one launch: integer unary + per-node max + integer edge weights (pygco converts the edge
     // weights on every call, the down-weight factor changes with the model)
     if ((rc = launch_quantise(r->d_logp, r->n, ctx->K, r->d_dwf, tol, ctx->uprec, r->d_unary, r->d_rowmax, r->d_blist,
-                              r->bcap, r->d_absmax + 1, r->E > 0 ? r->d_edge_w : nullptr, r->E, ctx->wprec,
+                              r->bcap, r->d_absmax + 1, r->E > 0 ? r->d_edge_w.get() : nullptr, r->E, ctx->wprec,
                               r->d_edge_wi, ctx->sm_count, r->stream)) != PHMRF_OK)
         return rc;
     r->have_unary = true;
@@ -778,11 +698,11 @@ int phmrf_quantise(phmrf_region *r, double dwf_in, double tol, int32_t *unary_i3
                                        r->stream));
         PHMRF_CUDA(cudaStreamSynchronize(r->stream));
     }
-    if ((rc = launch_publish(r->d_small + kSmDwf, r->d_dwf, 2, false, r->stream)) != PHMRF_OK) return rc;
-    if ((rc = launch_publish(r->d_small + kSmAbsmax, r->d_absmax, 2, false, r->stream)) != PHMRF_OK) return rc;
+    if ((rc = launch_publish(r->small.dev + kSmDwf, r->d_dwf, 2, false, r->stream)) != PHMRF_OK) return rc;
+    if ((rc = launch_publish(r->small.dev + kSmAbsmax, r->d_absmax, 2, false, r->stream)) != PHMRF_OK) return rc;
     PHMRF_CUDA(cudaStreamSynchronize(r->stream));
-    std::memcpy(dwf2, r->h_small + kSmDwf, sizeof(dwf2));
-    nb = r->h_small[kSmAbsmax + 1];
+    std::memcpy(dwf2, r->small.host + kSmDwf, sizeof(dwf2));
+    nb = r->small.host[kSmAbsmax + 1];
     if (dwf_out) *dwf_out = dwf2[0];
     if (n_boundary) *n_boundary = (int64_t)nb;
     if (boundary_idx && boundary_cap > 0 && nb > 0) {
@@ -790,8 +710,7 @@ int phmrf_quantise(phmrf_region *r, double dwf_in, double tol, int32_t *unary_i3
         if (m > r->bcap) m = r->bcap;
         PHMRF_CUDA(cudaMemcpy(boundary_idx, r->d_blist, sizeof(long long) * m, cudaMemcpyDeviceToHost));
     }
-    if (V_i32_out)  // K*K values: host (numpy: (V * _SMOOTH_COST_PRECISION).astype(intc))
-        for (int i = 0; i < K * K; ++i) V_i32_out[i] = (int32_t)(ctx->V[i] * ctx->sprec);
+    if (V_i32_out) smooth_costs_i32(ctx, V_i32_out);
     return PHMRF_OK;
 }
 
@@ -800,14 +719,8 @@ int phmrf_set_labels(phmrf_region *r, const int32_t *labels_window) {
     if (!r || !labels_window) return PHMRF_E_INVALID;
     int rc = set_device(r->ctx);
     if (rc) return rc;
-    PHMRF_CUDA(cudaMemcpyAsync(r->d_labels, labels_window, sizeof(int32_t) * r->n_window, cudaMemcpyHostToDevice,
-                               r->stream));
-    // range check on the device (a host loop over 4e7 labels costs more than the copy)
     long long first_bad = -1;
-    if ((rc = launch_check_labels(r->d_labels, r->n_window, r->ctx->K, r->d_badlabel, r->stream)) != PHMRF_OK) return rc;
-    if ((rc = launch_publish(r->d_small + kSmBadLabel, r->d_badlabel, 1, false, r->stream)) != PHMRF_OK) return rc;
-    PHMRF_CUDA(cudaStreamSynchronize(r->stream));
-    first_bad = (long long)r->h_small[kSmBadLabel];
+    if ((rc = upload_labels(r, labels_window, r->n_window, &first_bad)) != PHMRF_OK) return rc;
     if (first_bad >= 0) {
         r->have_labels = false;
         set_error("phmrf_set_labels: label out of range at node " + std::to_string(first_bad));
@@ -901,7 +814,7 @@ static int estep_enqueue(phmrf_region *r, int estimate_type, bool want_post, boo
             a.grid_kind = r->grid_kind;
         } else {
             if (!r->d_nbr_g) {
-                if ((rc = dev_alloc(r, &r->d_nbr_g, (int64_t)r->W * r->ld)) != PHMRF_OK) return rc;
+                if ((rc = r->d_nbr_g.alloc((int64_t)r->W * r->ld, &r->bytes)) != PHMRF_OK) return rc;
                 r->g_weighted = -1;
             }
             if (r->g_weighted != weighted || r->g_beta != ctx->beta) {
@@ -924,22 +837,16 @@ int phmrf_estep_stats(phmrf_region *r, int estimate_type, double *post_out, doub
                       double *cost_sums_out) {
     int rc = estep_enqueue(r, estimate_type, post_out != nullptr);
     if (rc) return rc;
-    phmrf_ctx *ctx = r->ctx;
-    const int K = ctx->K;
-    const int64_t len = phmrf_stats_len(ctx);
+    const int64_t len = phmrf_stats_len(r->ctx);
     std::vector<double> host((size_t)len);
     for (int attempt = 0; attempt < 2; ++attempt) {
         int flag = 0;
-        if (post_out && r->n > 0) {
-            double *aos = r->d_scratch + (int64_t)K * r->ld;
-            if ((rc = launch_soa_to_aos(r->d_scratch, aos, r->n, K, r->ld, r->stream)) != PHMRF_OK) return rc;
-            PHMRF_CUDA(cudaMemcpyAsync(post_out, aos, sizeof(double) * r->n * K, cudaMemcpyDeviceToHost, r->stream));
-        }
-        if ((rc = launch_publish(r->d_small + kSmStats, r->d_stats, (int)len, false, r->stream)) != PHMRF_OK) return rc;
-        if ((rc = launch_publish(r->d_small + kSmFlag, r->d_flags, 1, true, r->stream)) != PHMRF_OK) return rc;
+        if (post_out && (rc = enqueue_rows_download(r, post_out)) != PHMRF_OK) return rc;
+        if ((rc = launch_publish(r->small.dev + kSmStats, r->d_stats, (int)len, false, r->stream)) != PHMRF_OK) return rc;
+        if ((rc = launch_publish(r->small.dev + kSmFlag, r->d_flags, 1, true, r->stream)) != PHMRF_OK) return rc;
         PHMRF_CUDA(cudaStreamSynchronize(r->stream));
-        std::memcpy(host.data(), r->h_small + kSmStats, sizeof(double) * len);
-        flag = (int)(long long)r->h_small[kSmFlag];
+        std::memcpy(host.data(), r->small.host + kSmStats, sizeof(double) * len);
+        flag = (int)(long long)r->small.host[kSmFlag];
         if (!(flag & 1) || attempt == 1) break;
         // the pipeline kernel met a soft-max overflow (only reachable with extreme beta):
         // redo the region on the general kernel, which uses the exact maximum
@@ -953,13 +860,7 @@ int phmrf_estep_stats(phmrf_region *r, int estimate_type, double *post_out, doub
 int phmrf_pairwise_potential(phmrf_region *r, int estimate_type, double *pp_out) {
     if (!r || !pp_out) return PHMRF_E_INVALID;
     int rc = estep_enqueue(r, estimate_type, false, true);
-    if (rc) return rc;
-    const int K = r->ctx->K;
-    if (r->n > 0) {
-        double *aos = r->d_scratch + (int64_t)K * r->ld;
-        if ((rc = launch_soa_to_aos(r->d_scratch, aos, r->n, K, r->ld, r->stream)) != PHMRF_OK) return rc;
-        PHMRF_CUDA(cudaMemcpyAsync(pp_out, aos, sizeof(double) * r->n * K, cudaMemcpyDeviceToHost, r->stream));
-    }
+    if (rc || (rc = enqueue_rows_download(r, pp_out))) return rc;
     PHMRF_CUDA(cudaStreamSynchronize(r->stream));
     return PHMRF_OK;
 }
@@ -1006,32 +907,24 @@ int phmrf_graph_cut_swap(int device, int64_t n_sites, int32_t n_labels, const in
                 set_error("GCO (device swap) phmrf_graph_cut_swap: init label out of range");
                 return PHMRF_E_INVALID;
             }
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || device < 0 || device >= count) {
-        cudaGetLastError();
-        set_error("GCO (device swap) phmrf_graph_cut_swap: no such CUDA device (this library has no CPU fallback)");
-        return PHMRF_E_CUDA;
-    }
-    PHMRF_CUDA(cudaSetDevice(device));
+    int rc = use_device(device, "GCO (device swap) phmrf_graph_cut_swap");
+    if (rc) return rc;
+    SwapScratch s;
+    DevBuf<int32_t> d_unary, d_labels, d_w;
+    DevBuf<long long> d_ids;
+    if ((rc = swap_scratch_alloc(s, n_sites, n_edges, n_labels)) || (rc = d_unary.alloc(n_sites * n_labels)) ||
+        (rc = d_labels.alloc(n_sites)) || (rc = d_w.alloc(n_edges)) || (rc = d_ids.alloc(2 * n_edges)))
+        return rc;
     cudaStream_t st = nullptr;
     PHMRF_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    SwapScratch s;
-    int32_t *d_unary = nullptr, *d_w = nullptr, *d_labels = nullptr;
-    long long *d_ids = nullptr;
-    int rc = swap_scratch_alloc(s, n_sites, n_edges, n_labels);
     const size_t nu = sizeof(int32_t) * (size_t)n_sites * n_labels;
-    if (rc == PHMRF_OK &&
-        (cudaMalloc((void **)&d_unary, nu) != cudaSuccess ||
-         cudaMalloc((void **)&d_labels, sizeof(int32_t) * n_sites) != cudaSuccess ||
-         cudaMalloc((void **)&d_w, sizeof(int32_t) * (n_edges > 0 ? n_edges : 1)) != cudaSuccess ||
-         cudaMalloc((void **)&d_ids, sizeof(long long) * 2 * (n_edges > 0 ? n_edges : 1)) != cudaSuccess ||
-         cudaMemcpyAsync(d_unary, unary, nu, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-         (n_edges > 0 &&
-          (cudaMemcpyAsync(d_w, edge_w, sizeof(int32_t) * n_edges, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-           cudaMemcpyAsync(d_ids, edge_ids, sizeof(long long) * 2 * n_edges, cudaMemcpyHostToDevice, st) !=
-               cudaSuccess)) ||
-         (init_labels ? cudaMemcpyAsync(d_labels, init_labels, sizeof(int32_t) * n_sites, cudaMemcpyHostToDevice, st)
-                      : cudaMemsetAsync(d_labels, 0, sizeof(int32_t) * n_sites, st)) != cudaSuccess))
+    if (cudaMemcpyAsync(d_unary, unary, nu, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        (n_edges > 0 &&
+         (cudaMemcpyAsync(d_w, edge_w, sizeof(int32_t) * n_edges, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+          cudaMemcpyAsync(d_ids, edge_ids, sizeof(long long) * 2 * n_edges, cudaMemcpyHostToDevice, st) !=
+              cudaSuccess)) ||
+        (init_labels ? cudaMemcpyAsync(d_labels, init_labels, sizeof(int32_t) * n_sites, cudaMemcpyHostToDevice, st)
+                     : cudaMemsetAsync(d_labels, 0, sizeof(int32_t) * n_sites, st)) != cudaSuccess)
         rc = cuda_fail(cudaGetLastError(), "graph cut upload", __FILE__, __LINE__);
     if (rc == PHMRF_OK) rc = swap_graph_from_edges(s, d_ids, st);
     if (rc == PHMRF_OK) rc = swap_run(s, d_unary, d_w, smooth, d_labels, n_iter, energy_out, energy_before_out, st);
@@ -1039,12 +932,7 @@ int phmrf_graph_cut_swap(int device, int64_t n_sites, int32_t n_labels, const in
         (cudaMemcpyAsync(labels_out, d_labels, sizeof(int32_t) * n_sites, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
          cudaStreamSynchronize(st) != cudaSuccess))
         rc = cuda_fail(cudaGetLastError(), "graph cut download", __FILE__, __LINE__);
-    cudaStreamSynchronize(st);
-    cudaFree(d_unary);
-    cudaFree(d_labels);
-    cudaFree(d_w);
-    cudaFree(d_ids);
-    swap_scratch_free(s);
+    cudaStreamSynchronize(st);  // before the buffers go
     cudaStreamDestroy(st);
     return rc;
 }
@@ -1069,25 +957,18 @@ int phmrf_region_graph_cut(phmrf_region *r, const int32_t *init_labels, int32_t 
     if (rc) return rc;
     const int K = ctx->K;
     if (!r->cut) {
-        r->cut = new SwapScratch();
-        rc = swap_scratch_alloc(*r->cut, r->n, r->E, K);
-        if (rc == PHMRF_OK) rc = swap_graph_from_ell(*r->cut, r->d_nbr_id, r->W, r->ld, r->stream);
-        if (rc == PHMRF_OK) PHMRF_CUDA(cudaStreamSynchronize(r->stream));
-        if (rc != PHMRF_OK) {
-            swap_scratch_free(*r->cut);
-            delete r->cut;
-            r->cut = nullptr;
+        std::unique_ptr<SwapScratch> cut(new SwapScratch());
+        if ((rc = swap_scratch_alloc(*cut, r->n, r->E, K)) ||
+            (rc = swap_graph_from_ell(*cut, r->d_nbr_id, r->W, r->ld, r->stream)))
             return rc;
-        }
-        r->bytes += r->cut->bytes;
+        PHMRF_CUDA(cudaStreamSynchronize(r->stream));
+        r->bytes += cut->bytes;
+        r->cut = std::move(cut);
     }
     r->have_labels = false;
     if (init_labels) {
-        PHMRF_CUDA(cudaMemcpyAsync(r->d_labels, init_labels, sizeof(int32_t) * r->n, cudaMemcpyHostToDevice, r->stream));
-        if ((rc = launch_check_labels(r->d_labels, r->n, K, r->d_badlabel, r->stream)) != PHMRF_OK) return rc;
-        if ((rc = launch_publish(r->d_small + kSmBadLabel, r->d_badlabel, 1, false, r->stream)) != PHMRF_OK) return rc;
-        PHMRF_CUDA(cudaStreamSynchronize(r->stream));
-        const long long first_bad = (long long)r->h_small[kSmBadLabel];
+        long long first_bad = -1;
+        if ((rc = upload_labels(r, init_labels, r->n, &first_bad)) != PHMRF_OK) return rc;
         if (first_bad >= 0) {
             set_error("GCO (device swap) phmrf_region_graph_cut: init label out of range at node " + std::to_string(first_bad));
             return PHMRF_E_INVALID;
@@ -1096,7 +977,7 @@ int phmrf_region_graph_cut(phmrf_region *r, const int32_t *init_labels, int32_t 
         PHMRF_CUDA(cudaMemsetAsync(r->d_labels, 0, sizeof(int32_t) * r->n, r->stream));
     }
     std::vector<int32_t> V((size_t)K * K);  // as phmrf_quantise hands V_i32 to the host cut
-    for (int i = 0; i < K * K; ++i) V[i] = (int32_t)(ctx->V[i] * ctx->sprec);
+    smooth_costs_i32(ctx, V.data());
     if ((rc = swap_run(*r->cut, r->d_unary, r->d_edge_wi, V.data(), r->d_labels, n_iter, energy_out, energy_before_out,
                        r->stream)) != PHMRF_OK)
         return rc;
@@ -1122,31 +1003,19 @@ int phmrf_grid_edges(int device, const double *X, int n_features, int kind, int6
         set_error("phmrf_grid_edges: invalid arguments (kind 0/1, num_neighbor 8/4, n_edges from phmrf_grid_edge_count)");
         return PHMRF_E_INVALID;
     }
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || device < 0 || device >= count) {
-        cudaGetLastError();
-        set_error("phmrf_grid_edges: no such CUDA device (this library has no CPU fallback)");
-        return PHMRF_E_CUDA;
-    }
-    PHMRF_CUDA(cudaSetDevice(device));
+    int rc = use_device(device, "phmrf_grid_edges");
+    if (rc) return rc;
     const int64_t n = kind == 1 ? n2 * (n2 + 1) / 2 : n1 * n2;
-    double *dX = nullptr, *dE = nullptr;
-    PHMRF_CUDA(cudaMalloc((void **)&dX, sizeof(double) * n * n_features));
-    if (cudaMalloc((void **)&dE, sizeof(double) * 3 * (n_edges > 0 ? n_edges : 1)) != cudaSuccess) {
-        cudaFree(dX);
-        return cuda_fail(cudaGetLastError(), "cudaMalloc(edge list)", __FILE__, __LINE__);
-    }
-    int rc = PHMRF_OK;
+    DevBuf<double> dX, dE;
+    if ((rc = dX.alloc(n * n_features)) || (rc = dE.alloc(3 * n_edges))) return rc;
     if (cudaMemcpy(dX, X, sizeof(double) * n * n_features, cudaMemcpyHostToDevice) != cudaSuccess)
-        rc = cuda_fail(cudaGetLastError(), "upload X", __FILE__, __LINE__);
-    if (rc == PHMRF_OK && n_edges > 0)
-        rc = launch_grid_edges(dX, kind, n1, n2, num_neighbor, n_features, n, n_edges, dE, nullptr);
-    if (rc == PHMRF_OK && n_edges > 0 &&
+        return cuda_fail(cudaGetLastError(), "upload X", __FILE__, __LINE__);
+    if (n_edges > 0 && (rc = launch_grid_edges(dX, kind, n1, n2, num_neighbor, n_features, n, n_edges, dE, nullptr)))
+        return rc;
+    if (n_edges > 0 &&
         cudaMemcpy(edge_list_out, dE, sizeof(double) * 3 * n_edges, cudaMemcpyDeviceToHost) != cudaSuccess)
-        rc = cuda_fail(cudaGetLastError(), "download edge list", __FILE__, __LINE__);
-    cudaFree(dX);
-    cudaFree(dE);
-    return rc;
+        return cuda_fail(cudaGetLastError(), "download edge list", __FILE__, __LINE__);
+    return PHMRF_OK;
 }
 
 }  // extern "C"

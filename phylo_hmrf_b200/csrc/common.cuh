@@ -21,6 +21,51 @@ void count_launch(int n = 1);
         if (_e != cudaSuccess) return ::phmrf::cuda_fail(_e, #expr, __FILE__, __LINE__); \
     } while (0)
 
+// The owners of the library's device and mapped memory: nothing else frees it.
+
+// One cudaMalloc of T, freed by the destructor.  Converts to T * so that launch sites read as with a raw pointer.
+template <typename T>
+class DevBuf {
+  public:
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p_(o.p_) { o.p_ = nullptr; }
+    ~DevBuf() {
+        if (p_) cudaFree(p_);
+    }
+    // Frees what it holds and allocates `count` elements (at least one); adds their size to *bytes when given.
+    int alloc(int64_t count, int64_t *bytes = nullptr) {
+        if (p_) cudaFree(p_);
+        p_ = nullptr;
+        if (count <= 0) count = 1;
+        PHMRF_CUDA(cudaMalloc((void **)&p_, sizeof(T) * (size_t)count));
+        if (bytes) *bytes += (int64_t)sizeof(T) * count;
+        return PHMRF_OK;
+    }
+    T *get() const { return p_; }
+    operator T *() const { return p_; }
+
+  private:
+    T *p_ = nullptr;
+};
+
+// One pinned host block of 64-bit words mapped into the device (cudaHostAllocMapped | Portable): kernels store
+// small results through `dev` (launch_publish) and the host reads them through `host` after a stream sync.
+struct MappedBuf {
+    unsigned long long *host = nullptr, *dev = nullptr;
+    MappedBuf() = default;
+    MappedBuf(const MappedBuf &) = delete;
+    MappedBuf &operator=(const MappedBuf &) = delete;
+    ~MappedBuf() {
+        if (host) cudaFreeHost(host);
+    }
+    int alloc(size_t words) {
+        PHMRF_CUDA(cudaHostAlloc((void **)&host, words * sizeof(unsigned long long),
+                                 cudaHostAllocMapped | cudaHostAllocPortable));
+        PHMRF_CUDA(cudaHostGetDevicePointer((void **)&dev, host, 0));
+        return PHMRF_OK;
+    }
+};
+
 // Per-state emission parameters as the kernels consume them (built on the host from the
 // Cholesky factor): z = Wh*x - ch with Wh = sqrt(1/2)*L^-1 (lower triangular), ch = Wh*mu,
 // and logp = -(hc + sum z^2) with hc = (d*ln(2pi) + logdet)/2.  Stored as the stream the
@@ -152,18 +197,17 @@ int launch_fwd_factor(double2 *fwd, long long count, double beta, int weighted, 
 struct SwapScratch {
     int64_t n = 0, E = 0, bytes = 0;
     int K = 0;
-    long long *start = nullptr;                                       // [n+1]
-    long long *nbr = nullptr, *eid = nullptr, *rev = nullptr, *rcap = nullptr;  // [2E]
-    int32_t *wslot = nullptr;                                         // [2E] integer edge weight per slot
-    long long *act = nullptr, *var = nullptr;                         // active sites; site -> compact index or -1
-    long long *excess = nullptr, *inflow = nullptr, *tcap = nullptr;  // per compact index
-    int *h = nullptr;                                                 // heights
-    int32_t *V = nullptr;                                             // [K*K]
-    long long *ctl = nullptr;                                         // control words
-    unsigned long long *h_map = nullptr, *d_map = nullptr;            // their host-mapped copy
+    DevBuf<long long> start;                  // [n+1]
+    DevBuf<long long> nbr, eid, rev, rcap;    // [2E]
+    DevBuf<int32_t> wslot;                    // [2E] integer edge weight per slot
+    DevBuf<long long> act, var;               // active sites; site -> compact index or -1
+    DevBuf<long long> excess, inflow, tcap;   // per compact index
+    DevBuf<int> h;                            // heights
+    DevBuf<int32_t> V;                        // [K*K]
+    DevBuf<long long> ctl;                    // control words
+    MappedBuf map;                            // their host-mapped copy
 };
 int swap_scratch_alloc(SwapScratch &s, int64_t n, int64_t E, int K);
-void swap_scratch_free(SwapScratch &s);
 // the graph from a device edge list [E,2] (0 <= id1 < id2 < n)
 int swap_graph_from_edges(SwapScratch &s, const long long *edge_ids, cudaStream_t st);
 // the graph from a region's neighbour slots [W][ld] (-1 = empty), filled from an edge list sorted by (id1, id2)

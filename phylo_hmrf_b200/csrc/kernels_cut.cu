@@ -336,33 +336,24 @@ __global__ void apply_kernel(int64_t n_act, const long long *act, const int *h, 
     }
 }
 
-template <typename T>
-int salloc(SwapScratch &s, T **p, int64_t count) {
-    if (count <= 0) count = 1;
-    PHMRF_CUDA(cudaMalloc((void **)p, sizeof(T) * (size_t)count));
-    s.bytes += (int64_t)sizeof(T) * count;
-    return PHMRF_OK;
-}
-
 int exclusive_scan(const long long *in, long long *out, int64_t count, cudaStream_t st) {
     size_t bytes = 0;
     PHMRF_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, in, out, count, st));
-    void *tmp = nullptr;
-    PHMRF_CUDA(cudaMalloc(&tmp, bytes));
-    cudaError_t e = cub::DeviceScan::ExclusiveSum(tmp, bytes, in, out, count, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    cudaFree(tmp);
-    PHMRF_CUDA(e);
+    DevBuf<unsigned char> tmp;
+    int rc = tmp.alloc((int64_t)bytes);
+    if (rc) return rc;
+    PHMRF_CUDA(cub::DeviceScan::ExclusiveSum(tmp.get(), bytes, in, out, count, st));
+    PHMRF_CUDA(cudaStreamSynchronize(st));
     count_launch();
     return PHMRF_OK;
 }
 
 // the control words as the host sees them after the stream drains
 int read_ctl(SwapScratch &s, cudaStream_t st, long long *out) {
-    int rc = launch_publish(s.d_map, s.ctl, kCtlWords, false, st);
+    int rc = launch_publish(s.map.dev, s.ctl, kCtlWords, false, st);
     if (rc) return rc;
     PHMRF_CUDA(cudaStreamSynchronize(st));
-    for (int w = 0; w < kCtlWords; ++w) out[w] = (long long)s.h_map[w];
+    for (int w = 0; w < kCtlWords; ++w) out[w] = (long long)s.map.host[w];
     return PHMRF_OK;
 }
 
@@ -441,32 +432,19 @@ int swap_scratch_alloc(SwapScratch &s, int64_t n, int64_t E, int K) {
     s.E = E;
     s.K = K;
     const int64_t slots = 2 * E;
+    int64_t *b = &s.bytes;
     int rc;
-    if ((rc = salloc(s, &s.start, n + 1)) || (rc = salloc(s, &s.nbr, slots)) || (rc = salloc(s, &s.eid, slots)) ||
-        (rc = salloc(s, &s.rev, slots)) || (rc = salloc(s, &s.rcap, slots)) || (rc = salloc(s, &s.wslot, slots)) ||
-        (rc = salloc(s, &s.act, n)) || (rc = salloc(s, &s.var, n + 1)) || (rc = salloc(s, &s.excess, n + 1)) ||
-        (rc = salloc(s, &s.inflow, n)) || (rc = salloc(s, &s.tcap, n)) || (rc = salloc(s, &s.h, n)) ||
-        (rc = salloc(s, &s.V, (int64_t)K * K)) || (rc = salloc(s, &s.ctl, kCtlWords)))
+    if ((rc = s.start.alloc(n + 1, b)) || (rc = s.nbr.alloc(slots, b)) || (rc = s.eid.alloc(slots, b)) ||
+        (rc = s.rev.alloc(slots, b)) || (rc = s.rcap.alloc(slots, b)) || (rc = s.wslot.alloc(slots, b)) ||
+        (rc = s.act.alloc(n, b)) || (rc = s.var.alloc(n + 1, b)) || (rc = s.excess.alloc(n + 1, b)) ||
+        (rc = s.inflow.alloc(n, b)) || (rc = s.tcap.alloc(n, b)) || (rc = s.h.alloc(n, b)) ||
+        (rc = s.V.alloc((int64_t)K * K, b)) || (rc = s.ctl.alloc(kCtlWords, b)))
         return rc;
-    void *h = nullptr, *d = nullptr;
-    PHMRF_CUDA(cudaHostAlloc(&h, kCtlWords * sizeof(unsigned long long), cudaHostAllocMapped | cudaHostAllocPortable));
-    s.h_map = static_cast<unsigned long long *>(h);
-    PHMRF_CUDA(cudaHostGetDevicePointer(&d, h, 0));
-    s.d_map = static_cast<unsigned long long *>(d);
-    return PHMRF_OK;
-}
-
-void swap_scratch_free(SwapScratch &s) {
-    cudaFree(s.start); cudaFree(s.nbr); cudaFree(s.eid); cudaFree(s.rev); cudaFree(s.rcap); cudaFree(s.wslot);
-    cudaFree(s.act); cudaFree(s.var); cudaFree(s.excess); cudaFree(s.inflow); cudaFree(s.tcap); cudaFree(s.h);
-    cudaFree(s.V); cudaFree(s.ctl);
-    if (s.h_map) cudaFreeHost(s.h_map);
-    cudaGetLastError();
-    s = SwapScratch();
+    return s.map.alloc(kCtlWords);
 }
 
 int swap_graph_from_edges(SwapScratch &s, const long long *edge_ids, cudaStream_t st) {
-    unsigned long long *deg = reinterpret_cast<unsigned long long *>(s.excess);  // [n+1] counts, then cursors
+    unsigned long long *deg = reinterpret_cast<unsigned long long *>(s.excess.get());  // [n+1] counts, then cursors
     PHMRF_CUDA(cudaMemsetAsync(deg, 0, sizeof(long long) * (s.n + 1), st));
     if (s.E > 0) LAUNCH(edge_degree_kernel, s.E, edge_ids, s.E, deg);
     int rc = exclusive_scan(s.excess, s.start, s.n + 1, st);

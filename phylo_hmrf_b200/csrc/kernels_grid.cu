@@ -294,25 +294,22 @@ long long grid_edge_count(int kind, long long n1, long long n2, int nn) {
 int launch_grid_edges(const double *X_dev, int kind, long long n1, long long n2, int nn, int D, long long n,
                       long long n_edges, double *edge_list_dev, cudaStream_t s) {
     Grid g{kind, n1, n2, nn};
-    int *counts = nullptr;
-    long long *offsets = nullptr;
-    void *tmp = nullptr;
+    DevBuf<int> counts;
+    DevBuf<long long> offsets;
+    DevBuf<unsigned char> tmp;
     size_t tmp_bytes = 0;
-    PHMRF_CUDA(cudaMalloc((void **)&counts, sizeof(int) * (n + 1)));
-    PHMRF_CUDA(cudaMalloc((void **)&offsets, sizeof(long long) * (n + 1)));
+    int rc;
+    if ((rc = counts.alloc(n + 1)) || (rc = offsets.alloc(n + 1))) return rc;
     const int grid = (int)((n + 255) / 256 < 148 * 16 ? (n + 255) / 256 : 148 * 16);
     grid_count_kernel<<<grid, 256, 0, s>>>(g, n, counts);
     count_launch();
-    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts, offsets, n, s);
-    PHMRF_CUDA(cudaMalloc(&tmp, tmp_bytes));
-    cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, counts, offsets, n, s);
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts.get(), offsets.get(), n, s);
+    if ((rc = tmp.alloc((int64_t)tmp_bytes))) return rc;
+    cub::DeviceScan::ExclusiveSum(tmp.get(), tmp_bytes, counts.get(), offsets.get(), n, s);
     count_launch();
     grid_fill_kernel<<<grid, 256, 0, s>>>(g, n, D, X_dev, offsets, edge_list_dev);
     count_launch();
     cudaError_t e = cudaStreamSynchronize(s);
-    cudaFree(counts);
-    cudaFree(offsets);
-    cudaFree(tmp);
     (void)n_edges;
     if (e != cudaSuccess) return cuda_fail(e, "grid edge kernels", __FILE__, __LINE__);
     PHMRF_CUDA(cudaGetLastError());
@@ -335,41 +332,26 @@ int launch_band_graph(const double *Xw_dev, int kind, long long n1, long long n2
     Band b{win_start, own_start, own_end};
     const long long n_own = own_end - own_start;
     const int grid = (int)((n_window + 255) / 256 < 148 * 16 ? (n_window + 255) / 256 : 148 * 16);
+    // both calls: the edges each window node starts, and their exclusive scan (the first edge of each node)
+    DevBuf<int> counts;
+    DevBuf<long long> offsets;
+    DevBuf<unsigned char> tmp;
+    size_t tmp_bytes = 0;
+    int rc;
+    if ((rc = counts.alloc(n_window + 1)) || (rc = offsets.alloc(n_window + 1))) return rc;
+    PHMRF_CUDA(cudaMemsetAsync(counts, 0, sizeof(int) * (n_window + 1), s));
+    band_count_kernel<<<grid, 256, 0, s>>>(g, b, n_window, counts);
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts.get(), offsets.get(), n_window + 1, s);
+    if ((rc = tmp.alloc((int64_t)tmp_bytes))) return rc;
+    cub::DeviceScan::ExclusiveSum(tmp.get(), tmp_bytes, counts.get(), offsets.get(), n_window + 1, s);
     if (ids_dev == nullptr) {
-        int *counts = nullptr;
-        long long *offsets = nullptr;
-        void *tmp = nullptr;
-        size_t tmp_bytes = 0;
-        PHMRF_CUDA(cudaMalloc((void **)&counts, sizeof(int) * (n_window + 1)));
-        PHMRF_CUDA(cudaMalloc((void **)&offsets, sizeof(long long) * (n_window + 1)));
-        PHMRF_CUDA(cudaMemsetAsync(counts, 0, sizeof(int) * (n_window + 1), s));
-        band_count_kernel<<<grid, 256, 0, s>>>(g, b, n_window, counts);
-        cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts, offsets, n_window + 1, s);
-        PHMRF_CUDA(cudaMalloc(&tmp, tmp_bytes));
-        cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, counts, offsets, n_window + 1, s);
         count_launch(2);
         long long total = 0;
         PHMRF_CUDA(cudaMemcpyAsync(&total, offsets + n_window, sizeof(long long), cudaMemcpyDeviceToHost, s));
         PHMRF_CUDA(cudaStreamSynchronize(s));
         *n_edges = total;
-        // keep the offsets for the fill call: stash them behind the caller's back is not possible
-        // with plain pointers, so the fill call recomputes them (two cheap kernels)
-        cudaFree(counts);
-        cudaFree(offsets);
-        cudaFree(tmp);
         return PHMRF_OK;
     }
-    int *counts = nullptr;
-    long long *offsets = nullptr;
-    void *tmp = nullptr;
-    size_t tmp_bytes = 0;
-    PHMRF_CUDA(cudaMalloc((void **)&counts, sizeof(int) * (n_window + 1)));
-    PHMRF_CUDA(cudaMalloc((void **)&offsets, sizeof(long long) * (n_window + 1)));
-    PHMRF_CUDA(cudaMemsetAsync(counts, 0, sizeof(int) * (n_window + 1), s));
-    band_count_kernel<<<grid, 256, 0, s>>>(g, b, n_window, counts);
-    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts, offsets, n_window + 1, s);
-    PHMRF_CUDA(cudaMalloc(&tmp, tmp_bytes));
-    cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, counts, offsets, n_window + 1, s);
     PHMRF_CUDA(cudaMemsetAsync(wmax_bits, 0, sizeof(unsigned long long), s));
     band_fill_kernel<<<grid, 256, 0, s>>>(g, b, n_window, D, Xw_dev, beta1, offsets, ids_dev, w_dev, wmax_bits);
     if (n_own > 0) {
@@ -378,9 +360,6 @@ int launch_band_graph(const double *Xw_dev, int kind, long long n1, long long n2
     }
     count_launch(4);
     cudaError_t e = cudaStreamSynchronize(s);
-    cudaFree(counts);
-    cudaFree(offsets);
-    cudaFree(tmp);
     if (e != cudaSuccess) return cuda_fail(e, "band graph kernels", __FILE__, __LINE__);
     PHMRF_CUDA(cudaGetLastError());
     return PHMRF_OK;

@@ -293,13 +293,6 @@ __global__ void interleave_kernel(const double *__restrict__ plane, int64_t coun
         img[e * d + c] = plane[e];
 }
 
-struct DevBuf {
-    void *p = nullptr;
-    ~DevBuf() { cudaFree(p); }
-    template <typename T>
-    T *as() { return static_cast<T *>(p); }
-};
-
 inline int grid_for(int64_t count, int cap = 148 * 16) {
     const int64_t b = (count + 255) / 256;
     return (int)(b < 1 ? 1 : (b < cap ? b : cap));
@@ -318,21 +311,20 @@ extern "C" int phmrf_prep_normalise(int device, double *x, int64_t n, int d, dou
         return PHMRF_E_INVALID;
     }
     PHMRF_CUDA(cudaSetDevice(device));
-    DevBuf dx, dmn, dmx, dmm;
-    PHMRF_CUDA(cudaMalloc(&dx.p, sizeof(double) * n * d));
-    PHMRF_CUDA(cudaMalloc(&dmn.p, sizeof(unsigned long long) * d));
-    PHMRF_CUDA(cudaMalloc(&dmx.p, sizeof(unsigned long long) * d));
-    PHMRF_CUDA(cudaMalloc(&dmm.p, sizeof(double) * 2 * d));
-    PHMRF_CUDA(cudaMemcpy(dx.p, x, sizeof(double) * n * d, cudaMemcpyHostToDevice));
-    PHMRF_CUDA(cudaMemset(dmn.p, 0xff, sizeof(unsigned long long) * d));
-    PHMRF_CUDA(cudaMemset(dmx.p, 0, sizeof(unsigned long long) * d));
+    DevBuf<double> dx, dmm;
+    DevBuf<unsigned long long> dmn, dmx;
+    int rc;
+    if ((rc = dx.alloc(n * d)) || (rc = dmn.alloc(d)) || (rc = dmx.alloc(d)) || (rc = dmm.alloc(2 * d))) return rc;
+    PHMRF_CUDA(cudaMemcpy(dx, x, sizeof(double) * n * d, cudaMemcpyHostToDevice));
+    PHMRF_CUDA(cudaMemset(dmn, 0xff, sizeof(unsigned long long) * d));
+    PHMRF_CUDA(cudaMemset(dmx, 0, sizeof(unsigned long long) * d));
     dim3 g1((unsigned)grid_for(n, 148 * 4), (unsigned)d);
-    colminmax_kernel<<<g1, 256>>>(dx.as<double>(), n, d, dmn.as<unsigned long long>(), dmx.as<unsigned long long>());
+    colminmax_kernel<<<g1, 256>>>(dx, n, d, dmn, dmx);
     count_launch();
     PHMRF_CUDA(cudaGetLastError());
     std::vector<unsigned long long> hmn(d), hmx(d);
-    PHMRF_CUDA(cudaMemcpy(hmn.data(), dmn.p, sizeof(unsigned long long) * d, cudaMemcpyDeviceToHost));
-    PHMRF_CUDA(cudaMemcpy(hmx.data(), dmx.p, sizeof(unsigned long long) * d, cudaMemcpyDeviceToHost));
+    PHMRF_CUDA(cudaMemcpy(hmn.data(), dmn, sizeof(unsigned long long) * d, cudaMemcpyDeviceToHost));
+    PHMRF_CUDA(cudaMemcpy(hmx.data(), dmx, sizeof(unsigned long long) * d, cudaMemcpyDeviceToHost));
     std::vector<double> mm(2 * (size_t)d), lo(d), hi(d);
     for (int c = 0; c < d; ++c) {
         memcpy(&mm[2 * c], &hmn[c], 8);
@@ -348,11 +340,11 @@ extern "C" int phmrf_prep_normalise(int device, double *x, int64_t n, int d, dou
     if (*x_min < 0) *x_min = median(lo);
     if (*x_max < 0) *x_max = median(hi);
     if (colminmax_out) memcpy(colminmax_out, mm.data(), sizeof(double) * 2 * d);
-    PHMRF_CUDA(cudaMemcpy(dmm.p, mm.data(), sizeof(double) * 2 * d, cudaMemcpyHostToDevice));
-    rescale_kernel<<<grid_for(n * d), 256>>>(dx.as<double>(), n, d, dmm.as<double>(), *x_min, *x_max, log1p);
+    PHMRF_CUDA(cudaMemcpy(dmm, mm.data(), sizeof(double) * 2 * d, cudaMemcpyHostToDevice));
+    rescale_kernel<<<grid_for(n * d), 256>>>(dx, n, d, dmm, *x_min, *x_max, log1p);
     count_launch();
     PHMRF_CUDA(cudaGetLastError());
-    PHMRF_CUDA(cudaMemcpy(x, dx.p, sizeof(double) * n * d, cudaMemcpyDeviceToHost));
+    PHMRF_CUDA(cudaMemcpy(x, dx, sizeof(double) * n * d, cudaMemcpyDeviceToHost));
     return PHMRF_OK;
 }
 
@@ -368,8 +360,11 @@ extern "C" int phmrf_prep_region_image(int device, const double *value, const in
     PHMRF_CUDA(cudaSetDevice(device));
     const int64_t npix = n1 * n2;
     const int64_t n_nodes = kind == 1 ? n1 * (n1 + 1) / 2 : npix;
-    DevBuf dval, dpos, dplane, df0, df1, ddata, dimg, dbad, dgw, dtmp;
-    int lw = 0;
+    DevBuf<double> dval, dplane, ddata, dimg, dgw, dtmp;
+    DevBuf<int64_t> dpos;
+    DevBuf<float> df0, df1;
+    DevBuf<int> dbad;
+    int lw = 0, rc;
     if (filter_mode == 2 && sigma > 0) {
         // scipy.ndimage._filters._gaussian_kernel1d: radius int(4 sigma + 0.5), exp(-x^2 / (2 sigma^2)) normalised
         lw = (int)(4.0 * sigma + 0.5);
@@ -381,47 +376,41 @@ extern "C" int phmrf_prep_region_image(int device, const double *value, const in
             tot += gw[x + lw];
         }
         for (auto &v : gw) v /= tot;
-        PHMRF_CUDA(cudaMalloc(&dgw.p, sizeof(double) * gw.size()));
-        PHMRF_CUDA(cudaMemcpy(dgw.p, gw.data(), sizeof(double) * gw.size(), cudaMemcpyHostToDevice));
-        PHMRF_CUDA(cudaMalloc(&dtmp.p, sizeof(double) * npix));
+        if ((rc = dgw.alloc((int64_t)gw.size())) || (rc = dtmp.alloc(npix))) return rc;
+        PHMRF_CUDA(cudaMemcpy(dgw, gw.data(), sizeof(double) * gw.size(), cudaMemcpyHostToDevice));
     }
     // species are independent: the (latency-bound, one CTA per plane) hole fill runs for a batch of
     // planes at once, as many as fit a 48 GB budget
     int batch = (int)std::max<int64_t>(1, std::min<int64_t>(d, (int64_t)48e9 / (int64_t)(sizeof(double) * npix)));
-    PHMRF_CUDA(cudaMalloc(&dval.p, sizeof(double) * n * d));
-    PHMRF_CUDA(cudaMalloc(&dpos.p, sizeof(int64_t) * 2 * n));
-    PHMRF_CUDA(cudaMalloc(&dplane.p, sizeof(double) * npix * batch));
-    PHMRF_CUDA(cudaMalloc(&ddata.p, sizeof(double) * n_nodes * d));
-    PHMRF_CUDA(cudaMalloc(&dbad.p, sizeof(int)));
-    if (filter_mode == 0 && niter > 0) {
-        PHMRF_CUDA(cudaMalloc(&df0.p, sizeof(float) * npix));
-        PHMRF_CUDA(cudaMalloc(&df1.p, sizeof(float) * npix));
-    }
-    if (image_out) PHMRF_CUDA(cudaMalloc(&dimg.p, sizeof(double) * npix * d));
-    PHMRF_CUDA(cudaMemcpy(dval.p, value, sizeof(double) * n * d, cudaMemcpyHostToDevice));
-    PHMRF_CUDA(cudaMemcpy(dpos.p, pos, sizeof(int64_t) * 2 * n, cudaMemcpyHostToDevice));
-    PHMRF_CUDA(cudaMemset(dbad.p, 0, sizeof(int)));
+    if ((rc = dval.alloc(n * d)) || (rc = dpos.alloc(2 * n)) || (rc = dplane.alloc(npix * batch)) ||
+        (rc = ddata.alloc(n_nodes * d)) || (rc = dbad.alloc(1)))
+        return rc;
+    if (filter_mode == 0 && niter > 0 && ((rc = df0.alloc(npix)) || (rc = df1.alloc(npix)))) return rc;
+    if (image_out && (rc = dimg.alloc(npix * d))) return rc;
+    PHMRF_CUDA(cudaMemcpy(dval, value, sizeof(double) * n * d, cudaMemcpyHostToDevice));
+    PHMRF_CUDA(cudaMemcpy(dpos, pos, sizeof(int64_t) * 2 * n, cudaMemcpyHostToDevice));
+    PHMRF_CUDA(cudaMemset(dbad, 0, sizeof(int)));
     const dim3 g2((unsigned)((n2 + 255) / 256), (unsigned)(n1 < 4096 ? n1 : 4096));
     for (int c0 = 0; c0 < d; c0 += batch) {
         const int nb = std::min(batch, d - c0);
-        PHMRF_CUDA(cudaMemsetAsync(dplane.p, 0, sizeof(double) * npix * nb));
+        PHMRF_CUDA(cudaMemsetAsync(dplane, 0, sizeof(double) * npix * nb));
         for (int q = 0; q < nb; ++q)
-            scatter_kernel<<<grid_for(n), 256>>>(dval.as<double>(), dpos.as<int64_t>(), n, d, c0 + q, start1, start2, n1,
-                                                 n2, kind == 1, dplane.as<double>() + (int64_t)q * npix, dbad.as<int>());
+            scatter_kernel<<<grid_for(n), 256>>>(dval, dpos, n, d, c0 + q, start1, start2, n1, n2, kind == 1,
+                                                 dplane + (int64_t)q * npix, dbad);
         count_launch(nb);
         {
-            const int rc_fill = launch_holefill(dplane.as<double>(), npix, nb, n1, n2, kind == 1, nullptr);
+            const int rc_fill = launch_holefill(dplane, npix, nb, n1, n2, kind == 1, nullptr);
             if (rc_fill != PHMRF_OK) return rc_fill;
         }
         for (int q = 0; q < nb; ++q) {
             const int c = c0 + q;
-            double *plane = dplane.as<double>() + (int64_t)q * npix;
+            double *plane = dplane + (int64_t)q * npix;
             if (kind == 1) {
                 mirror_kernel<<<grid_for(npix), 256>>>(plane, n1);
                 count_launch();
             }
             if (filter_mode == 0 && niter > 0) {
-                float *a = df0.as<float>(), *b = df1.as<float>();
+                float *a = df0, *b = df1;
                 to_f32_kernel<<<grid_for(npix), 256>>>(plane, a, npix);
                 for (int it = 0; it < niter; ++it) {
                     diffuse_kernel<<<g2, 256>>>(a, b, n1, n2, (float)kappa, (float)gamma);
@@ -431,26 +420,26 @@ extern "C" int phmrf_prep_region_image(int device, const double *value, const in
                 count_launch(niter + 2);
             }
             if (filter_mode == 2 && sigma > 0) {  // axis 0 then axis 1, like scipy
-                gauss1d_kernel<<<g2, 256>>>(plane, dtmp.as<double>(), n1, n2, 0, dgw.as<double>(), lw);
-                gauss1d_kernel<<<g2, 256>>>(dtmp.as<double>(), plane, n1, n2, 1, dgw.as<double>(), lw);
+                gauss1d_kernel<<<g2, 256>>>(plane, dtmp, n1, n2, 0, dgw, lw);
+                gauss1d_kernel<<<g2, 256>>>(dtmp, plane, n1, n2, 1, dgw, lw);
                 count_launch(2);
             }
-            flatten_kernel<<<g2, 256>>>(plane, n1, n2, kind, d, c, ddata.as<double>());
+            flatten_kernel<<<g2, 256>>>(plane, n1, n2, kind, d, c, ddata);
             count_launch();
             if (image_out) {
-                interleave_kernel<<<grid_for(npix), 256>>>(plane, npix, d, c, dimg.as<double>());
+                interleave_kernel<<<grid_for(npix), 256>>>(plane, npix, d, c, dimg);
                 count_launch();
             }
         }
         PHMRF_CUDA(cudaGetLastError());
     }
     int bad = 0;
-    PHMRF_CUDA(cudaMemcpy(&bad, dbad.p, sizeof(int), cudaMemcpyDeviceToHost));
+    PHMRF_CUDA(cudaMemcpy(&bad, dbad, sizeof(int), cudaMemcpyDeviceToHost));
     if (bad) {
         set_error("phmrf_prep_region_image: a bin pair lies outside the region window");
         return PHMRF_E_INVALID;
     }
-    PHMRF_CUDA(cudaMemcpy(data_out, ddata.p, sizeof(double) * n_nodes * d, cudaMemcpyDeviceToHost));
-    if (image_out) PHMRF_CUDA(cudaMemcpy(image_out, dimg.p, sizeof(double) * npix * d, cudaMemcpyDeviceToHost));
+    PHMRF_CUDA(cudaMemcpy(data_out, ddata, sizeof(double) * n_nodes * d, cudaMemcpyDeviceToHost));
+    if (image_out) PHMRF_CUDA(cudaMemcpy(image_out, dimg, sizeof(double) * npix * d, cudaMemcpyDeviceToHost));
     return PHMRF_OK;
 }

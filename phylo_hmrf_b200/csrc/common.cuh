@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <limits>
 #include <string>
 
 #include "../../include/phmrf.h"
@@ -112,11 +113,13 @@ int launch_fill(double *p, double v, int64_t count, cudaStream_t s);
 int launch_publish(unsigned long long *dst_mapped, const void *src, int count, bool src32, cudaStream_t s);
 // rows of the log-likelihood matrix: K rounded up to the 8-state tiles of the pipeline kernel.  The
 // padding rows keep their values for the lifetime of a region: row K of an odd K holds kLogpPad (the
-// pipeline evaluates states in pairs: exp(-1e6 - shift) is a zero weight), the rows from the next even
-// number on hold 0.0 -- the pipeline never evaluates them, and the bulk copy then drops a zero WEIGHT
-// for them straight into the soft-max buffer the statistics product reads.
+// pipeline evaluates states in pairs: exp(-inf - shift) lands on its exp's lower clamp, e^-704, for ANY
+// shift -- a finite pad such as -1e6 outweighs the real states of a node whose log-likelihoods lie near or
+// below it), the rows from the next even number on hold 0.0 -- the pipeline never evaluates them, and the
+// bulk copy then drops a zero WEIGHT for them straight into the soft-max buffer the statistics product
+// reads.  Every other reader of the log-likelihood stops at row K - 1.
 __host__ __device__ inline int logp_rows(int K) { return (K + 7) / 8 * 8; }
-constexpr double kLogpPad = -1.0e6;
+constexpr double kLogpPad = -std::numeric_limits<double>::infinity();
 int launch_logp_init(double *logp, int64_t ld, int K, cudaStream_t s);
 // dwf = max(absmax_u, wmax*vmax) + 1e-10 unless dwf_in > 0; written to *dwf_dev.
 int launch_dwf(const unsigned long long *absmax_bits, double wmax, double vmax, double dwf_in, double *dwf_dev,

@@ -52,8 +52,9 @@ def _data(seed, B, d, K):
 
 
 def test_more_than_40_states_general_multipass(ph):
+    # d = 9: one pass of the general kernel holds 6 k-tiles of 5 states, so K = 45 takes two passes
     from phylo_hmrf_b200 import synth
-    X, e, w, means, covars = _data(1, 45, 6, 45)
+    X, e, w, means, covars = _data(1, 45, 9, 45)
     lab = np.random.default_rng(1).integers(0, 45, size=len(X))
     _check(ph, X, e, w, means, covars, synth.potts(45, 1.0), lab, 3, general=True)
 

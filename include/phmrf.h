@@ -177,6 +177,25 @@ int phmrf_estep_stats_async(phmrf_region *r, int estimate_type);
 /* Number of kernel launches this library has enqueued so far (bench "gpu_launches"). */
 int64_t phmrf_launch_count(void);
 
+/* ------------------------------------------------------------------ posterior summary --- */
+
+/* How confident the state map is at each owned node: the posterior over the K states that
+ * _compute_posteriors_graph forms (phylo_hmrf.py:334-355), post = softmax_k(logp - pp) with pp as
+ * phmrf_pairwise_potential defines it, for the resident log-likelihood and labels (halo included), reduced
+ * to four numbers per node instead of the dense [n_own,K] array:
+ *   map_state   int32  first k with the largest posterior (ties to the lowest index, like np.argmax)
+ *   map_prob    f64    that posterior
+ *   label_prob  f64    the posterior of the node's own label (the graph cut's state)
+ *   entropy     f64    -sum_k post_k ln post_k, in nats (a zero posterior contributes 0)
+ * phmrf_posterior_summary enqueues one kernel on the region's stream into a device buffer of 28 bytes per
+ * owned node (allocated at the first call, counted in phmrf_region_device_bytes) and copies nothing;
+ * PHMRF_E_STATE without a log-likelihood or labels.  phmrf_get_posterior_summary downloads the last summary
+ * into [n_own] host arrays (any pointer may be NULL) and synchronises; PHMRF_E_STATE before the first
+ * summary.  Neither changes what the E-step computes. */
+int phmrf_posterior_summary(phmrf_region *r, int estimate_type);
+int phmrf_get_posterior_summary(phmrf_region *r, int32_t *map_state, double *map_prob, double *label_prob,
+                                double *entropy);
+
 /* ------------------------------------------------------------------ graph cut ----------- */
 
 /* The alpha-beta swap of csrc/gco.cpp (phmrf_gco_cut_general_graph with algorithm PHMRF_GCO_SWAP) on the

@@ -56,6 +56,8 @@ SIGNATURES = {
     "phmrf_set_labels": (C.c_int, [_vp, _c_int32_p]),
     "phmrf_labels_argmin_unary": (C.c_int, [_vp, _c_int32_p]),
     "phmrf_estep_stats": (C.c_int, [_vp, C.c_int, _c_double_p, _c_double_p, _c_double_p]),
+    "phmrf_posterior_summary": (C.c_int, [_vp, C.c_int]),
+    "phmrf_get_posterior_summary": (C.c_int, [_vp, _c_int32_p, _c_double_p, _c_double_p, _c_double_p]),
     "phmrf_stats_device_ptr": (_vp, [_vp]),
     "phmrf_stats_len": (C.c_int64, [_vp]),
     "phmrf_absmax_device_ptr": (_vp, [_vp]),

@@ -20,7 +20,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "lib")
 OBJ = os.path.join(PKG, "build")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
-CU_SOURCES = ["api.cu", "kernels_a.cu", "kernels_b.cu", "kernels_b3.cu", "kernels_b3_d58.cu", "kernels_b3_d9c.cu", "kernels_grid.cu", "kernels_prep.cu", "kernels_cut.cu"]
+CU_SOURCES = ["api.cu", "kernels_a.cu", "kernels_b.cu", "kernels_b3.cu", "kernels_b3_d58.cu", "kernels_b3_d9c.cu", "kernels_grid.cu", "kernels_prep.cu", "kernels_cut.cu", "kernels_summary.cu"]
 
 
 def _nvcc() -> str:

@@ -91,6 +91,11 @@ def run(opts, device=0):
     graph_cut = os.environ.get("PHMRF_GRAPH_CUT", "host")
     if graph_cut not in ("host", "device"):
         raise SystemExit("PHMRF_GRAPH_CUT must be 'host' or 'device', not %r" % graph_cut)
+    # PHMRF_POSTERIOR_SUMMARY=1: also write the per-node summary of the posterior at the iteration whose labels
+    # are state_vec (posterior_ou_*.npz next to the .mat)
+    summary = os.environ.get("PHMRF_POSTERIOR_SUMMARY", "0")
+    if summary not in ("0", "1"):
+        raise SystemExit("PHMRF_POSTERIOR_SUMMARY must be 0 or 1, not %r" % summary)
     device, rank, world, td = _launch_context(device)
     run_id, K = int(opts.run_id), int(opts.num_states)
     cons_param = float(opts.cons_param)
@@ -133,13 +138,17 @@ def run(opts, device=0):
                       estimate_type=int(opts.estimate_type), max_iter=100, n_iter=5000, tol=1e-7, device=device,
                       graph_cut=graph_cut)
     filename = "%s/estimate_ou_%d_%.2f_%d_%s" % (output_path, run_id, cons_param, K, str(opts.annotation))
-    res = model.fit_accumulate_test(samples, len_vec, float(opts.threshold), filename, int(opts.miter))
+    extra = dict(posterior_summary=True) if summary == "1" else {}
+    res = model.fit_accumulate_test(samples, len_vec, float(opts.threshold), filename, int(opts.miter), **extra)
     params_vec1, params_vec2, params_vecList, iter_id1, iter_id2, cost_vec, state_vec = res
     mdict = {'state_vec': state_vec, 'len_vec': np.asarray(len_vec), 'params_vec1': params_vec1,
              'params_vec2': params_vec2, 'iter_id1': iter_id1, 'iter_id2': iter_id2, 'cost_vec': cost_vec}
     if rank == 0:
         os.makedirs(output_path, exist_ok=True)
         scipy.io.savemat("%s/estimate_ou_%d_%.2f_%d.mat" % (output_path, run_id, cons_param, K), mdict)
+        if summary == "1":
+            np.savez("%s/posterior_ou_%d_%.2f_%d.npz" % (output_path, run_id, cons_param, K),
+                     len_vec=np.asarray(len_vec), **model.posterior_summary_)
     model.close()
     return mdict
 

@@ -95,7 +95,10 @@ struct phmrf_region : RegionStream {
     DevBuf<long long> d_badlabel;  // [1] first out-of-range label index, -1 if none
     DevBuf<double> d_scratch;      // [K][ld] posteriors / AoS staging, allocated on demand
     int64_t scratch_elems = 0;
-    bool have_logp = false, have_unary = false, have_labels = false, have_rowmax = false;
+    // posterior summary (phmrf_posterior_summary): map_prob | label_prob | entropy [3][n] doubles, then map_state
+    // [n] int32 -- 28 bytes per owned node, allocated at the first call
+    DevBuf<double> d_summary;
+    bool have_logp = false, have_unary = false, have_labels = false, have_rowmax = false, have_summary = false;
     bool edges_sorted = true;   // edge list sorted by (id1, id2): the device cut numbers the edges from the slots
     std::unique_ptr<SwapScratch> cut;  // device graph cut, allocated at the first phmrf_region_graph_cut
     int64_t bytes = 0;
@@ -882,6 +885,81 @@ int phmrf_set_logprob(phmrf_region *r, const double *logprob) {
     r->have_logp = true;
     r->have_unary = false;
     r->have_rowmax = true;
+    return PHMRF_OK;
+}
+
+// ---------------------------------------------------------------- posterior summary
+int phmrf_posterior_summary(phmrf_region *r, int estimate_type) {
+    if (!r) {
+        set_error("phmrf_posterior_summary: null region");
+        return PHMRF_E_INVALID;
+    }
+    if (!r->have_logp || !r->have_labels) {
+        set_error("phmrf_posterior_summary: needs a log-likelihood and labels first");
+        return PHMRF_E_STATE;
+    }
+    phmrf_ctx *ctx = r->ctx;
+    int rc = set_device(ctx);
+    if (rc) return rc;
+    if (!r->d_summary) {
+        if ((rc = r->d_summary.alloc((28 * r->n + 7) / 8, &r->bytes)) != PHMRF_OK) return rc;
+    }
+    EstepArgs a{};
+    a.logp = r->d_logp;
+    a.labels = r->d_labels;
+    a.nbr_id = r->d_nbr_id;
+    a.nbr_w = r->d_nbr_w;
+    a.V = ctx->d_V;
+    a.beta = ctx->beta;
+    a.potts = ctx->potts ? 1 : 0;
+    a.n = r->n;
+    a.ld = r->ld;
+    a.own_offset = r->own_offset;
+    a.D = ctx->D;
+    a.K = ctx->K;
+    a.W = r->W;
+    a.estimate_type = estimate_type;
+    // grid-built regions: implicit neighbours and the forward weights (.x, set when the region is built)
+    a.fwd_wg = r->d_fwd;
+    a.ldw = r->ldw;
+    a.grid_kind = r->grid_kind;
+    a.grid_nn = r->grid_nn;
+    a.grid_n2 = r->grid_n2;
+    a.grid_rows = r->grid_rows;
+    a.own_start_gid = r->own_start_gid;
+    r->have_summary = false;
+    if ((rc = launch_posterior_summary(a, r->d_summary, reinterpret_cast<int32_t *>(r->d_summary + 3 * r->n),
+                                       ctx->sm_count, r->stream)) != PHMRF_OK)
+        return rc;
+    r->have_summary = true;
+    return PHMRF_OK;
+}
+
+int phmrf_get_posterior_summary(phmrf_region *r, int32_t *map_state, double *map_prob, double *label_prob,
+                                double *entropy) {
+    if (!r) {
+        set_error("phmrf_get_posterior_summary: null region");
+        return PHMRF_E_INVALID;
+    }
+    if (!r->have_summary) {
+        set_error("phmrf_get_posterior_summary: call phmrf_posterior_summary first");
+        return PHMRF_E_STATE;
+    }
+    int rc = set_device(r->ctx);
+    if (rc) return rc;
+    const int64_t n = r->n;
+    if (n > 0) {
+        std::lock_guard<std::mutex> turn(g_d2h_turn[r->ctx->device]);
+        double *const outs[3] = {map_prob, label_prob, entropy};
+        for (int q = 0; q < 3; ++q)
+            if (outs[q])
+                PHMRF_CUDA(cudaMemcpyAsync(outs[q], r->d_summary + q * n, sizeof(double) * n, cudaMemcpyDeviceToHost,
+                                           r->stream));
+        if (map_state)
+            PHMRF_CUDA(cudaMemcpyAsync(map_state, r->d_summary + 3 * n, sizeof(int32_t) * n, cudaMemcpyDeviceToHost,
+                                       r->stream));
+    }
+    PHMRF_CUDA(cudaStreamSynchronize(r->stream));
     return PHMRF_OK;
 }
 

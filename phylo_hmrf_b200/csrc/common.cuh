@@ -176,6 +176,10 @@ bool estep_bulk_supported(const EstepArgs &a);
 int launch_estep_bulk(const EstepArgs &a, int sm_count, cudaStream_t s);
 // Fold per-block partials into stats_out (defined in kernels_b.cu).
 int launch_estep_finalize(const double *partials, int n_blocks, int K, int D, double *stats_out, cudaStream_t s);
+// Posterior summary of the owned nodes (kernels_summary.cu) from the inputs of the E-step: out_d [3][n] =
+// map_prob | label_prob | entropy, out_state [n].  Reads the implicit grid when a.fwd_wg is set, else the
+// neighbour slots.
+int launch_posterior_summary(const EstepArgs &a, double *out_d, int32_t *out_state, int sm_count, cudaStream_t s);
 
 // ---- SURVEY 8(f-1): region edge lists on the GPU (kernels_grid.cu) ----------------------
 long long grid_edge_count(int kind, long long n1, long long n2, int nn);

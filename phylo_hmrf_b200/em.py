@@ -169,9 +169,39 @@ def band_window(kind, n1, n2, row0, row1):
     return int(starts[row0]), int(starts[row1]), int(starts[h0]), int(starts[h1])
 
 
-def run(model, X, len_vec, threshold, annotation, m_iter, lengths=None, n_threads=None):
+def empty_summary(n):
+    """Posterior summary of n nodes that have none: map_state -1, the probabilities and entropy NaN."""
+    return dict(map_state=np.full(n, -1, dtype=np.int32), map_prob=np.full(n, np.nan), label_prob=np.full(n, np.nan),
+                entropy=np.full(n, np.nan))
+
+
+def _gather_summary(model, len_vec, banded, label_owner, comm, n_samples):
+    """The posterior summary every rank computed for its pieces, on every rank: a whole region from the rank
+    that holds it, each band's owned rows from the band's rank."""
+    out = empty_summary(n_samples)
+    for rid in range(len(len_vec)):
+        s1, s2 = int(len_vec[rid][1]), int(len_vec[rid][2])
+        if rid in banded:
+            kind, n1, n2 = _geometry(len_vec[rid])
+            pieces = [(rank, bi) + band_window(kind, n1, n2, r0, r1)[:2] for bi, (rank, r0, r1) in enumerate(banded[rid])]
+        else:
+            pieces = [(label_owner[rid], None, 0, s2 - s1)]
+        for rank, bi, own0, own1 in pieces:
+            if rank == comm.rank:
+                got = model._summary_get(rid) if bi is None else model._band_summary_get(rid, bi)
+                for name, v in got.items():
+                    out[name][s1 + own0:s1 + own1] = v
+            for v in out.values():
+                v[s1 + own0:s1 + own1] = comm.broadcast_array(np.ascontiguousarray(v[s1 + own0:s1 + own1]), rank)
+    return out
+
+
+def run(model, X, len_vec, threshold, annotation, m_iter, lengths=None, n_threads=None, posterior_summary=False):
     """`fit_accumulate_test` (base.py:301-455): returns (params_vec, params_vec1, params_vecList,
-    iter_id1, iter_id2, cost_vec, t_labels)."""
+    iter_id1, iter_id2, cost_vec, t_labels).  posterior_summary: on every iteration that sets a new settled
+    best (the one whose labels become t_labels) the summary kernel runs on each of the rank's regions and bands
+    while their log-likelihood and labels are that iteration's; the pieces are gathered once, at the end, into
+    ``model.posterior_summary_``."""
     comm = Comm()
     if comm.rank == 0:
         model._init(X, lengths=lengths)
@@ -203,6 +233,7 @@ def run(model, X, len_vec, threshold, annotation, m_iter, lengths=None, n_thread
     params_settled = model.params_vec1.copy()
     params_trace = []
     t_labels = np.zeros(n_samples)
+    have_summary = False
 
     for it in range(m_iter):
         model._sync_model()
@@ -259,6 +290,14 @@ def run(model, X, len_vec, threshold, annotation, m_iter, lengths=None, n_thread
         if is_settled:
             params_settled = model.params_vec1.copy()
             t_labels = model.labels.copy()
+            if posterior_summary:
+                for rid in mine:
+                    model._summary_launch(rid)
+                for rid in sorted(banded):
+                    for bi, (rank, _, _) in enumerate(banded[rid]):
+                        if rank == comm.rank:
+                            model._band_summary_launch(rid, bi)
+                have_summary = True
         if stop:
             break
         if comm.rank == 0:
@@ -270,6 +309,10 @@ def run(model, X, len_vec, threshold, annotation, m_iter, lengths=None, n_thread
             s1, s2 = int(len_vec[rid][1]), int(len_vec[rid][2])
             for arr in (t_labels, model.labels, model.labels_local):
                 arr[s1:s2] = comm.broadcast_array(np.ascontiguousarray(arr[s1:s2]), label_owner[rid])
+    model.posterior_summary_ = None
+    if posterior_summary:
+        model.posterior_summary_ = (_gather_summary(model, len_vec, banded, label_owner, comm, n_samples)
+                                    if have_summary else empty_summary(n_samples))
     model.params_vec1 = params_settled.copy()
     model._ou_param_varied_constraint(params_best)
     return (params_best, params_settled, np.asarray(params_trace), history.best[0], history.best_settled[0],

@@ -210,6 +210,21 @@ class Region:
         check(_lib.lib().phmrf_estep_stats(self._h, int(estimate_type), dptr(post), dptr(flat), dptr(sums)))
         return unpack_stats(flat, K, d), sums, post
 
+    def posterior_summary(self, estimate_type):
+        """Enqueue the per-node summary of the posterior for the resident log-likelihood and labels
+        (phmrf_posterior_summary); nothing is copied until get_posterior_summary()."""
+        check(_lib.lib().phmrf_posterior_summary(self._h, int(estimate_type)))
+
+    def get_posterior_summary(self):
+        """-> dict of [n] arrays: map_state (int32), map_prob, label_prob, entropy (nats) of the last
+        posterior_summary()."""
+        n = self.n
+        out = dict(map_state=np.empty(n, dtype=np.int32), map_prob=np.empty(n), label_prob=np.empty(n),
+                   entropy=np.empty(n))
+        check(_lib.lib().phmrf_get_posterior_summary(self._h, i32ptr(out["map_state"]), dptr(out["map_prob"]),
+                                                     dptr(out["label_prob"]), dptr(out["entropy"])))
+        return out
+
     # ---- enqueue-only (bench)
     def emit_loglik_async(self):
         check(_lib.lib().phmrf_emit_loglik_async(self._h))

@@ -352,6 +352,27 @@ class phyloHMRF(object):
         m_queue.put((region_id, stats, labels, c[0], c[1], c[2], c[3]))
         return True
 
+    # ------------------------------------------------------------------ posterior summary
+    def posterior_summary(self, region_id):
+        """How confident the state map of a resident region is at each node, for the log-likelihood and labels
+        it currently holds (after _predict_posteriors): dict of [N_r] arrays map_state (int32), map_prob,
+        label_prob (posterior of the node's label) and entropy (nats); see phmrf_posterior_summary."""
+        self._summary_launch(region_id)
+        return self._summary_get(region_id)
+
+    def _summary_launch(self, rid):
+        self._regions[rid].posterior_summary(self.estimate_type)
+
+    def _summary_get(self, rid):
+        return self._regions[rid].get_posterior_summary()
+
+    def _band_summary_launch(self, rid, bi):
+        """The summary of one band's owned rows, for the band's current log-likelihood and label window."""
+        self._bands[(rid, bi)][0].posterior_summary(self.estimate_type)
+
+    def _band_summary_get(self, rid, bi):
+        return self._bands[(rid, bi)][0].get_posterior_summary()
+
     # ------------------------------------------------------------------ statistics helpers
     def _initialize_sufficient_statistics(self):
         """base.py:562-569 + phylo_hmrf.py:691-698."""
@@ -399,14 +420,18 @@ class phyloHMRF(object):
         if getattr(self, "finalize_fn", None) is not None:
             self.finalize_fn(self, params_vec)
 
-    def fit_accumulate_test(self, X, len_vec, threshold, annotation, m_iter, lengths=None, n_threads=None):
+    def fit_accumulate_test(self, X, len_vec, threshold, annotation, m_iter, lengths=None, n_threads=None,
+                            posterior_summary=False):
         """base.py:301-455 without fork: see `phylo_hmrf_b200.em` (iteration, cost aggregation with the
         N_r/N weights, convergence tests, best-iteration bookkeeping; regions on a thread pool; under
         `torchrun` the regions -- or the row bands of a region too large for one GPU -- are spread over
         the ranks).  Returns (params_vec, params_vec1, params_vecList, iter_id1, iter_id2, cost_vec,
-        t_labels)."""
+        t_labels).  posterior_summary=True also sets ``posterior_summary_``: the per-node summary of the
+        posterior (map_state, map_prob, label_prob, entropy over all n_samples) at the iteration whose labels
+        are t_labels."""
         from . import em
-        return em.run(self, X, len_vec, threshold, annotation, m_iter, lengths=lengths, n_threads=n_threads)
+        return em.run(self, X, len_vec, threshold, annotation, m_iter, lengths=lengths, n_threads=n_threads,
+                      posterior_summary=posterior_summary)
 
     # ------------------------------------------------------------------ row bands (SURVEY 8(e))
     def _prepare_bands(self, X, len_vec, banded, comm):
